@@ -7,6 +7,8 @@ the CausalConditionalDecoder estimator, then DAC-VAE decode, bf16 tensor-core op
   python bench.py --impl reference --gpus N --steps K --warmup W  (the reference algorithm on the host CPU cores)
 
 One JSON line on stdout (rank 0).  A step = one pass of the whole hot path over one batch of synthetic inputs.
+The inputs and weights are seeded, so ``--dump-outputs DIR`` (the waveforms of the last timed step as float32 .npy)
+lets two builds run with the same arguments be compared output for output.
 """
 import argparse
 import json
@@ -46,6 +48,24 @@ def emit(rec):
     _OUT.flush()
 
 
+DUMP_BYTES = 60 * 10 ** 6  # data written by --dump-outputs, all arrays together (below 64 MB with the .npy headers)
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as ``directory/<name>.npy`` in float32.  An array larger than its share of DUMP_BYTES is replaced
+    by a fixed, seeded sample of its elements (flattened; the same positions for the same shape), so that outputs of
+    two runs with the same arguments still line up element for element."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    budget = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > budget:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), budget))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -58,7 +78,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[2..4] / batch-1 latency legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 def config_of(a):
@@ -505,6 +531,9 @@ def run_b200(a):
     if ncu_range:
         torch.cuda.cudart().cudaProfilerStop()
     launches = native.launch_count() - l0
+    if a.dump_outputs and rank == 0:  # before any later call can reuse the output buffers
+        wav = out if world == 1 else torch.stack([out[uid] for uid in sorted(out)]).unsqueeze(1)
+        dump_outputs(a.dump_outputs, {"wav": wav})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -169,6 +169,22 @@ def test_header_is_plain_c(tmp_path):
     assert subprocess.run([str(exe)]).returncode == 0
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy per output, whole when it fits its share of the byte budget, else a seeded
+    sample of the same positions on every run."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 800)
+    small, large = torch.randn(2, 1, 10, dtype=torch.float64), torch.arange(1000.0).reshape(1, 1, 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"small": small, "large": large})
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float32 and s.shape == (2, 1, 10) and np.array_equal(s, small.float().numpy())
+    la, lb = np.load(tmp_path / "a" / "large.npy"), np.load(tmp_path / "b" / "large.npy")
+    assert la.dtype == np.float32 and 0 < la.size <= 100 and np.array_equal(la, lb)
+    assert np.all(np.diff(la) > 0) and np.all(la == np.round(la)) and la.max() < 1000  # distinct elements, in order
+
+
 def test_tblock_wide_ring_protocol():
     """The table-driven weight ring of csrc/tblock.cu (TBLOCK_WIDE_FF): no producer warp can alias a parity wait, and a
     randomised simulation of the real wait conditions neither overwrites an unconsumed box nor deadlocks."""
