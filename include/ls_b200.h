@@ -103,6 +103,12 @@ int32_t ls_dac_decode(ls_dac* h, const float* z, const int32_t* lengths, float* 
  * entries (ls_dac_create builds the decoder, the encoder, or both, from whatever the state dict holds). */
 int32_t ls_dac_encode(ls_dac* h, const float* audio, const float* noise, float* z, float* m, float* logs, int32_t B,
                       int32_t S, void* stream);
+/* ls_dac_encode for a right-padded batch of clips of different lengths.  lengths (DEVICE int32 [B], may be NULL =
+ * ls_dac_encode): valid latent frames per clip, clamped to [0, S/hop]; clip b is the samples [0, lengths[b]*hop) of
+ * its row and is encoded as if alone at that length (the samples after it are never read), noise is read over the
+ * same frames, and z, m, logs are zero from frame lengths[b] on (a length of 0 gives an all-zero item). */
+int32_t ls_dac_encode_lengths(ls_dac* h, const float* audio, const int32_t* lengths, const float* noise, float* z, float* m,
+                              float* logs, int32_t B, int32_t S, void* stream);
 
 /* ---- token -> mu front half (SURVEY section 8 f-1): CausalMaskedDiffWithXvec.inference up to the decoder call
  * (speech/cosyvoice/flow/flow.py:461-489): speaker-embedding normalise + affine, input embedding,

@@ -376,16 +376,21 @@ int32_t ls_dac_decode(ls_dac* h, const float* z, const int32_t* lengths, float* 
   });
 }
 
-int32_t ls_dac_encode(ls_dac* h, const float* audio, const float* noise, float* z, float* m, float* logs, int32_t B,
-                      int32_t S, void* stream) {
+int32_t ls_dac_encode_lengths(ls_dac* h, const float* audio, const int32_t* lengths, const float* noise, float* z, float* m,
+                              float* logs, int32_t B, int32_t S, void* stream) {
   return ls::guarded([&] {
     ls::require(h && audio && z && m && logs, "ls_dac_encode: null argument");
     ls::require(h->enc != nullptr || h->eng32 != nullptr, "ls_dac_encode: this handle holds no encoder weights",
                 LS_ERR_WEIGHTS);
     ls::SerialScope scope(h->serial, h->device(), (cudaStream_t)stream);
-    if (h->enc) h->enc->encode(audio, noise, z, m, logs, B, S, (cudaStream_t)stream);
-    else h->eng32->encode(audio, noise, z, m, logs, B, S, (cudaStream_t)stream);
+    if (h->enc) h->enc->encode(audio, lengths, noise, z, m, logs, B, S, (cudaStream_t)stream);
+    else h->eng32->encode(audio, lengths, noise, z, m, logs, B, S, (cudaStream_t)stream);
   });
+}
+
+int32_t ls_dac_encode(ls_dac* h, const float* audio, const float* noise, float* z, float* m, float* logs, int32_t B,
+                      int32_t S, void* stream) {
+  return ls_dac_encode_lengths(h, audio, nullptr, noise, z, m, logs, B, S, stream);
 }
 
 int32_t ls_synthesize_host(ls_flow* flow, ls_dac* dac, const float* mu_host, const float* mask_host,

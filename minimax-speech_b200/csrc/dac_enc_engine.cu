@@ -17,22 +17,33 @@
 namespace ls {
 namespace {
 
-// first convolution (1 -> C0, k = 7, pad 3) + LeakyReLU(0.1): x fp32 [B][S][C0] and snake(x) bf16 for the first unit
-__global__ void __launch_bounds__(128) enc_in_conv_kernel(const float* __restrict__ audio, const float* __restrict__ w,
+// first convolution (1 -> C0, k = 7, pad 3) + LeakyReLU(0.1): x fp32 [B][S][C0] and snake(x) bf16 for the first unit.
+// lengths (nullable, latent frames): item b is the samples [0, lengths[b] * hop) of its row; later samples are never
+// read (they count as the convolution's zero padding) and rows from there to S are written as zeros.
+__global__ void __launch_bounds__(128) enc_in_conv_kernel(const float* __restrict__ audio, const int* __restrict__ lengths,
+                                                          int hop, const float* __restrict__ w,
                                                           const float* __restrict__ bias, const float* __restrict__ alpha,
                                                           const float* __restrict__ ialpha, float* __restrict__ x,
                                                           __nv_bfloat16* __restrict__ sn, int S, int C0) {
   const int t = blockIdx.x * 128 + threadIdx.x;
   const int b = blockIdx.y;
   if (t >= S) return;
+  const int n_valid = lengths ? min(max(lengths[b], 0), S / hop) * hop : S;
+  float* xo = x + ((size_t)b * S + t) * C0;
+  __nv_bfloat16* so = sn + ((size_t)b * S + t) * C0;
+  if (t >= n_valid) {
+    for (int n = 0; n < C0; n += 4) {
+      *reinterpret_cast<float4*>(xo + n) = make_float4(0.f, 0.f, 0.f, 0.f);
+      *reinterpret_cast<uint2*>(so + n) = make_uint2(0u, 0u);
+    }
+    return;
+  }
   float a[7];
 #pragma unroll
   for (int k = 0; k < 7; ++k) {
     const int tt = t + k - 3;
-    a[k] = (tt >= 0 && tt < S) ? audio[(size_t)b * S + tt] : 0.f;
+    a[k] = (tt >= 0 && tt < n_valid) ? audio[(size_t)b * S + tt] : 0.f;
   }
-  float* xo = x + ((size_t)b * S + t) * C0;
-  __nv_bfloat16* so = sn + ((size_t)b * S + t) * C0;
   for (int n = 0; n < C0; n += 4) {
     float4 v;
     float* vv = &v.x;
@@ -55,13 +66,18 @@ __global__ void __launch_bounds__(128) enc_in_conv_kernel(const float* __restric
 }
 
 // y fp32 [B][L][latent] (conv3 + LeakyReLU(0.1) done) -> leaky_relu(0.01) -> en_conv_post (1x1, + LeakyReLU(0.1)) ->
-// split, clamp, reparameterise; outputs NCT [B][latent][L]
-__global__ void enc_post_kernel(const float* __restrict__ y, const float* __restrict__ w, const float* __restrict__ bias,
-                                const float* __restrict__ noise, float* __restrict__ z, float* __restrict__ m,
-                                float* __restrict__ logs, int L, int latent) {
+// split, clamp, reparameterise; outputs NCT [B][latent][L], zero at frames t >= lengths[b] (lengths nullable)
+__global__ void enc_post_kernel(const float* __restrict__ y, const int* __restrict__ lengths, const float* __restrict__ w,
+                                const float* __restrict__ bias, const float* __restrict__ noise, float* __restrict__ z,
+                                float* __restrict__ m, float* __restrict__ logs, int L, int latent) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;  // latent channel
   const int t = blockIdx.y, b = blockIdx.z;
   if (c >= latent) return;
+  if (lengths && t >= lengths[b]) {
+    const size_t o = ((size_t)b * latent + c) * L + t;
+    m[o] = 0.f, logs[o] = 0.f, z[o] = 0.f;
+    return;
+  }
   const float* yr = y + ((size_t)b * L + t) * latent;
   float am = bias[c], al = bias[latent + c];
   for (int k = 0; k < latent; ++k) {
@@ -244,8 +260,8 @@ const DacEncEngine::Plan& DacEncEngine::plan_for(int B, int S) {
   return ref;
 }
 
-void DacEncEngine::encode(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S,
-                          cudaStream_t s) {
+void DacEncEngine::encode(const float* audio, const int* lengths, const float* noise, float* z, float* m, float* logs,
+                          int B, int S, cudaStream_t s) {
   require(B > 0 && S > 0 && S % hop_ == 0, "audio length must be a positive multiple of the hop (pad first, model.py:455-462)");
   LS_CUDA(cudaSetDevice(device_));
   ensure_workspace(B, S, s);
@@ -256,22 +272,36 @@ void DacEncEngine::encode(const float* audio, const float* noise, float* z, floa
   void* sA = ws<void>(o_sA_);
   void* sB = ws<void>(o_sB_);
 
-  auto conv = [&](const CUtensorMap& a, const PackedLinear& w, long long rows, int dil, int pad, ConvGemmParams p) {
+  // Mixed lengths (lengths != nullptr, latent frames; clip b is the samples [0, n_b = lengths[b] * hop)): each clip is
+  // encoded as if alone at its own length.  A layer at rate r (rows per latent frame: hop / prod(strides[:i]) inside
+  // stage i, hop / prod(strides[:i+1]) for its downsampling conv, 1 for conv3) has L_b * r valid rows; every launch
+  // writes zeros to the rows of a computed tile past them and skips (leaves stale) the tiles starting at or past
+  // L_b * r + 64.  So the rows [L_b * r, L_b * r + 64) of every activation are zero (enc_in_conv_kernel zeroes the
+  // whole tail of stage 0), and no valid output reaches further: the conv7 at dilation 9 reads 27 rows past its own,
+  // the downsampling conv's pad of 1 view row is the input rows [L_b * r, L_b * r + s) with s < 64 -- the view stays
+  // aligned because n_b is a multiple of the hop -- and conv3 reads 1 row past.  Those zeros are exactly the zero
+  // padding the clip alone would see, so a valid output reads the same values either way; rows that are computed
+  // from stale data are past the valid length and written as zeros.
+  auto conv = [&](const CUtensorMap& a, const PackedLinear& w, long long rows, int rate, int dil, int pad, ConvGemmParams p) {
     p.B = B, p.M = (int)rows, p.N = w.N, p.block_n = w.block_n;
     p.taps = w.taps, p.dil = dil, p.pad = pad;
     p.kb_per_tap = (w.K + 63) / 64, p.kb_split = p.kb_per_tap;
-    p.lengths = nullptr, p.m_len_mul = 1, p.m_len_add = 0, p.skip_halo = 0;
+    if (lengths) p.lengths = lengths, p.m_len_mul = rate, p.m_len_add = 0, p.skip_halo = 64;
+    else p.lengths = nullptr, p.m_len_mul = 1, p.m_len_add = 0, p.skip_halo = 0;
     p.bias = w.bias, p.chan_mod = w.N, p.n_store = w.N;
-    p.out_ld = w.N, p.out_shift = 0, p.out_bstride = rows * w.N, p.out_alloc = rows * w.N, p.out_valid_mul = w.N;
+    p.out_ld = w.N, p.out_shift = 0, p.out_bstride = rows * w.N, p.out_alloc = rows * w.N;
+    p.out_valid_mul = lengths ? (long long)rate * w.N : w.N;
     p.k_true = w.K, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0;
     LS_CUDA(launch_conv_gemm(a, a, w.map, p, num_sms_, s));
   };
 
   count_launch();
-  enc_in_conv_kernel<<<dim3((S + 127) / 128, B), 128, 0, s>>>(audio, f32(in_w_), f32(in_b_), f32(stages_[0].unit[0].a0),
-                                                            f32(stages_[0].unit[0].ia0), x, ws<__nv_bfloat16>(o_sA_), S, dim0_);
+  enc_in_conv_kernel<<<dim3((S + 127) / 128, B), 128, 0, s>>>(audio, lengths, hop_, f32(in_w_), f32(in_b_),
+                                                            f32(stages_[0].unit[0].a0), f32(stages_[0].unit[0].ia0), x,
+                                                            ws<__nv_bfloat16>(o_sA_), S, dim0_);
   LS_CUDA(cudaGetLastError());
   long long rows = S;
+  int rate = hop_;
   static const int dils[3] = {1, 3, 9};
   for (size_t i = 0; i < stages_.size(); ++i) {
     const StageW& st = stages_[i];
@@ -280,7 +310,7 @@ void DacEncEngine::encode(const float* audio, const float* noise, float* z, floa
       {  // Snake (already applied) -> conv7 dilated -> LeakyReLU -> Snake
         ConvGemmParams p{};
         p.act = ACT_LRELU, p.out1 = sB, p.out1_mode = OUT1_SNAKE, p.p1_a = f32(u.a2), p.p1_b = f32(u.ia2);
-        conv(pl.st[i].d[j], u.conv7, rows, dils[j], 3 * dils[j], p);
+        conv(pl.st[i].d[j], u.conv7, rows, rate, dils[j], 3 * dils[j], p);
       }
       {  // conv1 -> LeakyReLU -> + x; secondary output = Snake of whatever consumes x next
         ConvGemmParams p{};
@@ -289,18 +319,18 @@ void DacEncEngine::encode(const float* audio, const float* noise, float* z, floa
         if (!last_unit) p.out0 = x, p.out0_dtype = OUT_F32;
         p.out1 = sA, p.out1_mode = OUT1_SNAKE;
         p.p1_a = f32(last_unit ? st.a_dn : st.unit[j + 1].a0), p.p1_b = f32(last_unit ? st.ia_dn : st.unit[j + 1].ia0);
-        conv(pl.st[i].b, u.conv1, rows, 1, 0, p);
+        conv(pl.st[i].b, u.conv1, rows, rate, 1, 0, p);
       }
     }
     {  // downsampling conv on the [rows/s][s*C] view: 3 taps, pad 1 -> LeakyReLU -> x of the next stage + its Snake
-      rows /= st.stride;
+      rows /= st.stride, rate /= st.stride;
       const bool last = i + 1 == stages_.size();
       ConvGemmParams p{};
       p.act = ACT_LRELU;
       if (!last) p.out0 = x, p.out0_dtype = OUT_F32;
       p.out1 = sB, p.out1_mode = OUT1_SNAKE;  // (sA is this launch's input: the Snake output goes to sB, then swaps)
       p.p1_a = f32(last ? final_alpha_ : stages_[i + 1].unit[0].a0), p.p1_b = f32(last ? final_ialpha_ : stages_[i + 1].unit[0].ia0);
-      conv(pl.st[i].down, st.down, rows, 1, 1, p);
+      conv(pl.st[i].down, st.down, rows, rate, 1, 1, p);
       // the next stage reads its Snake input from sA: copy (the tensors shrink by >= 2x per stage; this is a small
       // fraction of the stage's traffic)
       LS_CUDA(cudaMemcpyAsync(sA, sB, (size_t)B * rows * st.down.N * 2, cudaMemcpyDeviceToDevice, s));
@@ -309,11 +339,11 @@ void DacEncEngine::encode(const float* audio, const float* noise, float* z, floa
   {  // final Snake (applied) -> conv3 -> LeakyReLU(0.1): fp32 [B][L][latent]
     ConvGemmParams p{};
     p.act = ACT_LRELU, p.out0 = ws<float>(o_y_), p.out0_dtype = OUT_F32;
-    conv(pl.fin, final_, rows, 1, 1, p);
+    conv(pl.fin, final_, rows, rate, 1, 1, p);
   }
   count_launch();
-  enc_post_kernel<<<dim3((latent_ + 127) / 128, (unsigned)rows, B), 128, 0, s>>>(ws<float>(o_y_), f32(post_w_), f32(post_b_), noise, z, m,
-                                                                             logs, (int)rows, latent_);
+  enc_post_kernel<<<dim3((latent_ + 127) / 128, (unsigned)rows, B), 128, 0, s>>>(ws<float>(o_y_), lengths, f32(post_w_),
+                                                                             f32(post_b_), noise, z, m, logs, (int)rows, latent_);
   LS_CUDA(cudaGetLastError());
 }
 

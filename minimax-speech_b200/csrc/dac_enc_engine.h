@@ -13,8 +13,11 @@ class DacEncEngine {
  public:
   DacEncEngine(const Weights& w, int device);
   ~DacEncEngine();
-  // audio [B,1,S] fp32 (S a multiple of the hop) -> z, m, logs [B,latent,S/hop] fp32; noise nullable ([B,latent,S/hop])
-  void encode(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S, cudaStream_t s);
+  // audio [B,1,S] fp32 (S a multiple of the hop) -> z, m, logs [B,latent,S/hop] fp32; noise nullable ([B,latent,S/hop]).
+  // lengths (device int32 [B], nullable): latent frames per clip; clip b is encoded as if alone at lengths[b] * hop
+  // samples (the rest of its row is never read) and its outputs are zero from frame lengths[b] on.
+  void encode(const float* audio, const int* lengths, const float* noise, float* z, float* m, float* logs, int B, int S,
+              cudaStream_t s);
   int hop() const { return hop_; }
   int latent_dim() const { return latent_; }
   int device() const { return device_; }

@@ -894,14 +894,50 @@ float* DacEngineF32::residual_unit(const std::string& u, const float* x, int B, 
 }
 
 // DACVAE.encode (dac-vae/model.py:469-483) after Encoder (model.py:146-234); audio [B,1,S], S a multiple of the hop
-void DacEngineF32::encode(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S,
-                          cudaStream_t s) {
+void DacEngineF32::encode(const float* audio, const int* lengths, const float* noise, float* z, float* m, float* logs,
+                          int B, int S, cudaStream_t s) {
   require(!enc_rates_.empty(), "this handle holds no encoder weights", LS_ERR_WEIGHTS);
   int hop = 1;
   for (int r : enc_rates_) hop *= r;
   require(B > 0 && S > 0 && S % hop == 0, "audio length must be a positive multiple of the hop (pad first, model.py:455-462)");
   LS_CUDA(cudaSetDevice(device_));
   scratch_.reset();
+  if (!lengths) {
+    encode_dense(audio, noise, z, m, logs, B, S, s);
+    return;
+  }
+  // per-clip semantics: each clip is encoded alone at its own length (what a loop over the reference gives); the
+  // noise rows and the outputs have row stride L, so the clip's noise is gathered and its outputs scattered
+  const int L = S / hop;
+  const size_t row = (size_t)latent_ * L;
+  std::vector<int> h(B);
+  LS_CUDA(cudaMemcpyAsync(h.data(), lengths, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, s));
+  LS_CUDA(cudaStreamSynchronize(s));
+  for (float* o : {z, m, logs}) LS_CUDA(cudaMemsetAsync(o, 0, (size_t)B * row * sizeof(float), s));
+  for (int b = 0; b < B; ++b) {
+    const int n = h[b] < L ? h[b] : L;
+    if (n <= 0) continue;
+    scratch_.reset();
+    const size_t nd = (size_t)latent_ * n;
+    float* nz = noise ? scratch_.get(nd, s) : nullptr;
+    if (noise)
+      LS_CUDA(cudaMemcpy2DAsync(nz, (size_t)n * 4, noise + b * row, (size_t)L * 4, (size_t)n * 4, latent_,
+                                cudaMemcpyDeviceToDevice, s));
+    float* zd = scratch_.get(nd, s);
+    float* md = scratch_.get(nd, s);
+    float* ld = scratch_.get(nd, s);
+    encode_dense(audio + (size_t)b * S, nz, zd, md, ld, 1, n * hop, s);
+    const float* src[3] = {zd, md, ld};
+    float* dst[3] = {z, m, logs};
+    for (int k = 0; k < 3; ++k)
+      LS_CUDA(cudaMemcpy2DAsync(dst[k] + b * row, (size_t)L * 4, src[k], (size_t)n * 4, (size_t)n * 4, latent_,
+                                cudaMemcpyDeviceToDevice, s));
+  }
+}
+
+// audio [B,1,S] -> z, m, logs [B,latent,S/hop], all dense (the scratch memory is taken, not reset)
+void DacEngineF32::encode_dense(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S,
+                                cudaStream_t s) {
   int C = (int)w_.shape("encoder.block.0.0.weight")[0], len = S;
   float* x = scratch_.get((size_t)B * C * len, s);
   conv1d(audio, nullptr, w_.ptr("encoder.block.0.0.weight"), w_.ptr("encoder.block.0.0.bias"), x, nullptr, B, 1, len, C, 7, 1, 3,

@@ -75,8 +75,10 @@ class DacEngineF32 {
  public:
   DacEngineF32(const Weights& w, int device);
   void decode(const float* z, const int* lengths, float* wav, int B, int L, cudaStream_t s);
-  // DACVAE.encode (SURVEY section 8 f-3): audio [B,1,S] -> z, m, logs [B,latent,S/hop]; noise (nullable) [B,latent,S/hop]
-  void encode(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S, cudaStream_t s);
+  // DACVAE.encode (SURVEY section 8 f-3): audio [B,1,S] -> z, m, logs [B,latent,S/hop]; noise (nullable) [B,latent,S/hop];
+  // lengths (device int32 [B], nullable): latent frames per clip, each clip encoded alone, outputs zero past it
+  void encode(const float* audio, const int* lengths, const float* noise, float* z, float* m, float* logs, int B, int S,
+              cudaStream_t s);
   bool has_encoder() const { return !enc_rates_.empty(); }
   bool has_decoder() const { return !rates_.empty(); }
   int hop() const { return hop_; }
@@ -85,6 +87,7 @@ class DacEngineF32 {
 
  private:
   float* residual_unit(const std::string& u, const float* x, int B, int C, int len, int dil, cudaStream_t s);
+  void encode_dense(const float* audio, const float* noise, float* z, float* m, float* logs, int B, int S, cudaStream_t s);
   void decode_dense(const float* z, long long z_bstride, float* wav, long long wav_bstride, int B, int L, int L_alloc,
                     cudaStream_t s);
   int device_ = 0, latent_ = 80, hop_ = 1;

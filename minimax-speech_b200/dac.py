@@ -107,19 +107,30 @@ class DACVAEEncoder(nn.Module):
         return torch.nn.functional.pad(audio_data, (0, pad))
 
     @torch.inference_mode()
-    def encode(self, audio_data, noise=None):
+    def encode(self, audio_data, noise=None, lengths=None):
         """audio [B,1,S] (S a multiple of the hop) -> (z, m, logs).  ``noise`` ([B,latent,S/hop]) injects the sample
-        the reference draws with torch.randn_like; by default it is drawn here the same way."""
+        the reference draws with torch.randn_like; by default it is drawn here the same way.
+
+        ``lengths`` (optional list or tensor of B latent-frame counts in [1, S/hop]) encodes a right-padded batch of
+        clips of different lengths: clip b is ``audio_data[b, :, :lengths[b] * hop]`` and is encoded exactly as if
+        alone at that length (the samples after it are never read); z, m and logs are zero from frame lengths[b] on."""
         dev = audio_data.device
         if audio_data.dim() != 3 or audio_data.shape[1] != 1 or audio_data.shape[2] % self.hop_length or \
                 audio_data.shape[2] < self.hop_length:
             raise ValueError(f"audio must be [B, 1, S] with S a positive multiple of {self.hop_length}")
         B, _, S = audio_data.shape
+        L = S // self.hop_length
+        if lengths is not None:
+            host = torch.as_tensor(lengths).detach().cpu().reshape(-1)  # one copy per call: not a per-step call
+            if host.numel() != B or host.is_floating_point() or host.is_complex() or \
+                    bool(((host < 1) | (host > L)).any()):
+                raise ValueError(f"lengths must be {B} integer latent-frame counts in [1, {L}]")
+            lengths = host.to(device=dev, dtype=torch.int32)
         if noise is None:
-            noise = torch.randn(B, self.latent_dim, S // self.hop_length, device=dev)
-        elif tuple(noise.shape) != (B, self.latent_dim, S // self.hop_length):
+            noise = torch.randn(B, self.latent_dim, L, device=dev)
+        elif tuple(noise.shape) != (B, self.latent_dim, L):
             raise ValueError("noise must be [B, latent, S / hop]")
-        return self.handle(dev).encode(_as_f32(audio_data, dev), _as_f32(noise, dev))
+        return self.handle(dev).encode(_as_f32(audio_data, dev), _as_f32(noise, dev), lengths)
 
 
 def patch_reference_model(model):

@@ -15,6 +15,7 @@ OUT_NONE, OUT_F32, OUT_BF16 = range(3)
 OUT1_NONE, OUT1_LN, OUT1_COPY, OUT1_SNAKE = range(4)
 
 EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create", "ls_flow_create_fp16", "ls_flow_create_fp32", "ls_dac_create_fp32", "ls_dac_encode",
+           "ls_dac_encode_lengths",
            "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
            "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize",
@@ -103,6 +104,7 @@ def load():
         lib.ls_dac_hop_length.argtypes = [vp]
         lib.ls_dac_decode.argtypes = [vp, vp, vp, vp, i32, i32, vp]
         lib.ls_dac_encode.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, vp]
+        lib.ls_dac_encode_lengths.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, vp]
         lib.ls_front_create.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_front_create_fp32.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_front_destroy.argtypes = [vp]
@@ -355,12 +357,13 @@ class DacHandle:
         if h and _lib is not None:
             _lib.ls_dac_destroy(h)
 
-    def encode(self, audio, noise=None):
+    def encode(self, audio, noise=None, lengths=None):
+        """``lengths`` (optional device int32 [B]): valid latent frames per clip of a right-padded batch."""
         B, _, S = audio.shape
         latent, L = self.latent_dim, S // self.hop_length
         z, m, logs = (torch.empty(B, latent, L, device=audio.device, dtype=torch.float32) for _ in range(3))
-        check(load().ls_dac_encode(self._h, ptr(audio), ptr(noise), ptr(z), ptr(m), ptr(logs), B, S,
-                                   current_stream_ptr(self.device)), "ls_dac_encode")
+        check(load().ls_dac_encode_lengths(self._h, ptr(audio), ptr(lengths), ptr(noise), ptr(z), ptr(m), ptr(logs), B, S,
+                                           current_stream_ptr(self.device)), "ls_dac_encode_lengths")
         return z, m, logs
 
     def decode(self, z, lengths=None):

@@ -200,23 +200,67 @@ def latent_record(z, mu, logs, sample_rate, n_samples, n_padded, path):
             "original_path": path}
 
 
-def extract_latents(paths, load_audio, encoder, device, rank=0, world_size=1, save=True, generator=None):
-    """Encode this rank's share of ``paths`` one file at a time (like the reference) and write ``<stem>_latent2x.pt`` next
-    to each input.  ``load_audio(path) -> 1-D float tensor`` at ``encoder.sample_rate`` (the reference uses librosa, which
-    is not a dependency here).  Audio is clamped to [-1, 1] (:31) and right-padded to a multiple of the hop
-    (DACVAE.preprocess, model.py:455-462; the reference tool feeds the unpadded signal, so its last latent frame can
-    differ).  Returns the list of records (and output paths when saved)."""
+def plan_micro_batches(n_samples, max_batch_samples=None):
+    """Group items of ``n_samples`` (padded sample counts) into micro-batches of at most ``max_batch_samples`` padded
+    samples (batch size x longest item): items sorted by length (stable), filled greedily; an item longer than the
+    budget gets a batch of its own.  ``None``: one item per batch, in order.  Returns lists of item indices."""
+    if max_batch_samples is None:
+        return [[i] for i in range(len(n_samples))]
+    batches, cur = [], []
+    for i in sorted(range(len(n_samples)), key=lambda i: n_samples[i]):
+        if cur and (len(cur) + 1) * n_samples[i] > max_batch_samples:  # sorted: item i is the longest so far
+            batches.append(cur)
+            cur = []
+        cur.append(i)
+    if cur:
+        batches.append(cur)
+    return batches
+
+
+def extract_latents(paths, load_audio, encoder, device, rank=0, world_size=1, save=True, generator=None,
+                    max_batch_samples=None):
+    """Encode this rank's share of ``paths`` and write ``<stem>_latent2x.pt`` next to each input.
+    ``load_audio(path) -> 1-D float tensor`` at ``encoder.sample_rate`` (the reference uses librosa, which is not a
+    dependency here).  Audio is clamped to [-1, 1] (:31) and right-padded to a multiple of the hop (DACVAE.preprocess,
+    model.py:455-462; the reference tool feeds the unpadded signal, so its last latent frame can differ).
+
+    By default each file is encoded on its own (like the reference).  ``max_batch_samples`` encodes length-sorted
+    micro-batches of at most that many padded samples (batch size x longest file, see ``plan_micro_batches``) with
+    per-file ``lengths``, which gives every file the latents it gets alone; the share is loaded into host memory first.
+    Noise is drawn from ``generator`` in file order either way.  Returns the list of records (and output paths when
+    saved) in file order."""
     import os
     start, end = shard_files(len(paths), rank, world_size)
-    out = []
-    for path in paths[start:end]:
+    mine = paths[start:end]
+    padded, n_orig, noise = [], [], []
+    for path in mine:
         audio = torch.clamp(torch.as_tensor(load_audio(path), dtype=torch.float32).reshape(1, 1, -1), -1.0, 1.0)
-        n = audio.shape[-1]
-        padded = encoder.preprocess(audio)
-        L = padded.shape[-1] // encoder.hop_length
-        noise = torch.randn(1, encoder.latent_dim, L, generator=generator)
-        z, mu, logs = encoder.encode(padded.to(device), noise.to(device))
-        rec = latent_record(z, mu, logs, encoder.sample_rate, n, padded.shape[-1], path)
+        n_orig.append(audio.shape[-1])
+        padded.append(encoder.preprocess(audio))
+        L = padded[-1].shape[-1] // encoder.hop_length
+        noise.append(torch.randn(1, encoder.latent_dim, L, generator=generator))
+    recs = [None] * len(mine)
+    for batch in plan_micro_batches([a.shape[-1] for a in padded], max_batch_samples):
+        if len(batch) == 1:
+            i = batch[0]
+            z, mu, logs = encoder.encode(padded[i].to(device), noise[i].to(device))
+            recs[i] = latent_record(z, mu, logs, encoder.sample_rate, n_orig[i], padded[i].shape[-1], mine[i])
+            continue
+        s_max = max(padded[i].shape[-1] for i in batch)
+        audio = torch.zeros(len(batch), 1, s_max)
+        nz = torch.zeros(len(batch), encoder.latent_dim, s_max // encoder.hop_length)
+        lengths = []
+        for b, i in enumerate(batch):
+            audio[b, :, :padded[i].shape[-1]] = padded[i][0]
+            nz[b, :, :noise[i].shape[-1]] = noise[i][0]
+            lengths.append(noise[i].shape[-1])
+        z, mu, logs = (t.cpu() for t in encoder.encode(audio.to(device), nz.to(device), lengths=lengths))
+        for b, i in enumerate(batch):  # (copies: a saved view would carry the whole batch's storage)
+            n = lengths[b]
+            recs[i] = latent_record(z[b:b + 1, :, :n].clone(), mu[b:b + 1, :, :n].clone(), logs[b:b + 1, :, :n].clone(),
+                                    encoder.sample_rate, n_orig[i], padded[i].shape[-1], mine[i])
+    out = []
+    for path, rec in zip(mine, recs):
         if save:
             rec_path = os.path.splitext(path)[0] + "_latent2x.pt"
             torch.save(rec, rec_path)
