@@ -141,13 +141,18 @@ int32_t ls_speaker_encode(ls_speaker* h, const float* mel, float* embedding, int
 
 /* ---- S3 speech tokenizer (SURVEY section 8 f-4): S3TokenizerV2.quantize for clips of at most 30 s
  * (speech/tools/S3Tokenizer/s3tokenizer/model_v2.py:386-415) = AudioEncoderV2.forward (:320-351: two stride-2 convs,
- * FSMN attention blocks with rotary embedding :152-287) + FSQCodebook.encode (:97-112).  fp32 arithmetic only.
+ * FSMN attention blocks with rotary embedding :152-287) + FSQCodebook.encode (:97-112).  Two handle types share one call
+ * surface: ls_s3_create_fp32 (fp32 arithmetic on the CUDA cores) and ls_s3_create (bf16x3: every dense linear /
+ * convolution on the tensor cores as A_hi W_hi + A_lo W_hi + A_hi W_lo, hi = bf16(x), lo = bf16(x - hi), fp32
+ * accumulation; residual stream, LayerNorm, rotary, FSMN and attention in fp32 -- fp32-level error, since a token is a
+ * rounding decision; 716 MiB of weights at the shipped width against 470 MiB; encoder output rows past code_len[b] are zero).
  * mel [B,n_mels,T] (100 Hz log-mel, right-padded), mel_len [B] -> codes [B,T2] (ids < 3^8; frames past code_len[b] are
  * undefined, as in the reference), code_len [B]; T2 = ls_s3_code_frames(T); hidden (nullable): [B,T2,n_state], the
  * encoder output.  Weight names = the reference's state_dict keys; optional "rotary.cos" / "rotary.sin" [len][32] tables
  * (default: precompute_freqs_cis(64, 2048), model_v2.py:37-48).  All pointers are device pointers. */
 typedef struct ls_s3 ls_s3;
 int32_t ls_s3_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_s3** out);
+int32_t ls_s3_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_s3** out);
 void ls_s3_destroy(ls_s3* h);
 int32_t ls_s3_code_frames(int32_t T);
 int32_t ls_s3_quantize(ls_s3* h, const float* mel, const int32_t* mel_len, int32_t* codes, int32_t* code_len, float* hidden,

@@ -11,6 +11,7 @@
 #include "flow_engine.h"
 #include "front_engine.h"
 #include "profiler.h"
+#include "s3_engine.h"
 
 namespace ls {
 
@@ -185,7 +186,9 @@ struct ls_speaker {
 
 struct ls_s3 {
   ls::StreamSerial serial;
-  std::unique_ptr<ls::S3EngineF32> eng32;  // fp32 mode (the only one: tokens are rounding decisions)
+  int device() const { return eng ? eng->device() : eng32->device(); }
+  std::unique_ptr<ls::S3Engine> eng;       // bf16x3 tensor-core mode (fp32-level error: tokens are rounding decisions)
+  std::unique_ptr<ls::S3EngineF32> eng32;  // fp32 mode
 };
 
 extern "C" {
@@ -199,6 +202,15 @@ int32_t ls_s3_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_t d
     *out = h.release();
   });
 }
+int32_t ls_s3_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_s3** out) {
+  return ls::guarded([&] {
+    ls::require(weights && out && n_weights > 0, "ls_s3_create: null argument");
+    ls::Weights w(weights, n_weights);
+    auto h = std::make_unique<ls_s3>();
+    h->eng = std::make_unique<ls::S3Engine>(w, device);
+    *out = h.release();
+  });
+}
 void ls_s3_destroy(ls_s3* h) { delete h; }
 int32_t ls_s3_code_frames(int32_t T) {
   int t1 = 0, t2 = 0;
@@ -209,8 +221,9 @@ int32_t ls_s3_quantize(ls_s3* h, const float* mel, const int32_t* mel_len, int32
                        int32_t B, int32_t T, void* stream) {
   return ls::guarded([&] {
     ls::require(h && mel && mel_len && codes && code_len, "ls_s3_quantize: null argument");
-    ls::SerialScope scope(h->serial, h->eng32->device(), (cudaStream_t)stream);
-    h->eng32->quantize(mel, mel_len, codes, code_len, hidden, B, T, (cudaStream_t)stream);
+    ls::SerialScope scope(h->serial, h->device(), (cudaStream_t)stream);
+    if (h->eng) h->eng->quantize(mel, mel_len, codes, code_len, hidden, B, T, (cudaStream_t)stream);
+    else h->eng32->quantize(mel, mel_len, codes, code_len, hidden, B, T, (cudaStream_t)stream);
   });
 }
 

@@ -18,7 +18,7 @@ EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create
            "ls_dac_encode_lengths",
            "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
-           "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize",
+           "ls_s3_create", "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize",
            "ls_flow_destroy",
            "ls_flow_estimator_forward", "ls_flow_solve", "ls_dac_create", "ls_dac_destroy", "ls_dac_hop_length",
            "ls_dac_decode", "ls_synthesize_host", "ls_fsq_encode", "ls_mask_to_lengths", "ls_graph_create", "ls_graph_buffer",
@@ -116,6 +116,7 @@ def load():
         lib.ls_speaker_destroy.restype = None
         lib.ls_speaker_encode.argtypes = [vp, vp, vp, i32, i32, i32, vp]
         lib.ls_s3_create_fp32.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
+        lib.ls_s3_create.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_s3_destroy.argtypes = [vp]
         lib.ls_s3_destroy.restype = None
         lib.ls_s3_code_frames.argtypes = [i32]
@@ -301,16 +302,33 @@ class SpeakerHandle:
         return emb
 
 
-class S3Handle:
-    """Owns an ls_s3*: S3TokenizerV2 (fp32 mode)."""
+S3_PRECISIONS = ("fp32", "bf16x3")
 
-    def __init__(self, state_dict, device):
+
+def check_s3_precision(precision):
+    """The S3 tokenizer's precisions: "fp32" (CUDA cores) or "bf16x3" (tensor cores, every GEMM operand split into a bf16
+    high and low part: fp32-level error).  A token is a rounding decision, so plain 16-bit operands are refused."""
+    if precision in ("bf16", "fp16"):
+        raise ValueError(f"precision={precision!r} is not offered for the S3 tokenizer: 16-bit GEMM operands move the "
+                         "encoder output by about 5e-3 (rel-L2), and about 2 % of tokens change (801 of 820 identical "
+                         "with bf16 operands); use 'bf16x3' (tensor cores, fp32-level error) or 'fp32'")
+    if precision not in S3_PRECISIONS:
+        raise ValueError(f"precision must be 'fp32' or 'bf16x3', not {precision!r}")
+    return precision
+
+
+class S3Handle:
+    """Owns an ls_s3*: S3TokenizerV2, fp32 mode or the bf16x3 tensor-core mode."""
+
+    def __init__(self, state_dict, device, precision="fp32"):
         lib = load()
         self.device = torch.device(device)
+        self.precision = check_s3_precision(precision)
         arr, keep = tensor_table(state_dict)
         h = C.c_void_p()
+        create, name = (lib.ls_s3_create, "ls_s3_create") if precision == "bf16x3" else (lib.ls_s3_create_fp32, "ls_s3_create_fp32")
         with torch.cuda.device(self.device):
-            check(lib.ls_s3_create_fp32(arr, len(state_dict), self.device.index or 0, C.byref(h)), "ls_s3_create_fp32")
+            check(create(arr, len(state_dict), self.device.index or 0, C.byref(h)), name)
         self._h = h
         self.n_state = int(state_dict["encoder.conv1.weight"].shape[0])
 

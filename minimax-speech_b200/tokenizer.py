@@ -5,9 +5,12 @@ Drop-ins for ``s3tokenizer.model_v2.S3TokenizerV2`` (speech/tools/S3Tokenizer/s3
 (:290-351: two stride-2 convolutions, six FSMN-attention blocks with rotary embedding) and its quantizer head
 ``FSQCodebook`` / ``FSQVectorQuantization`` (:83-147: ``encode(hidden [B, T, dim]) -> int32 tokens [B, T]``), with the
 reference's parameter names, so a reference tokenizer checkpoint loads unchanged.  The tokens are the ids (vocabulary
-3^8 = 6561) the flow's ``input_embedding`` consumes.  fp32 arithmetic only (``ls_s3_quantize``): a token is a rounding
-decision.  Clips longer than 30 s take the reference's sliding-window path (model_v2.py:417-588: host-side windowing and
-merging around one batched device call).  Not built: the log-mel front end (utils.py ``log_mel_spectrogram``: an STFT with
+3^8 = 6561) the flow's ``input_embedding`` consumes.  A token is a rounding decision, so the arithmetic is fp32-level in
+both precisions of ``ls_s3_quantize``: ``"fp32"`` (default, CUDA cores) and ``"bf16x3"`` (tensor cores: every dense
+linear / convolution as A_hi W_hi + A_lo W_hi + A_hi W_lo with hi = bf16(x), lo = bf16(x - hi), fp32 accumulation;
+attention, FSMN, LayerNorm and the residual stream in fp32).  Plain bf16 / fp16 operands are refused.  Clips longer
+than 30 s take the reference's sliding-window path (model_v2.py:417-588: host-side windowing and merging around one
+batched device call).  Not built: the log-mel front end (utils.py ``log_mel_spectrogram``: an STFT with
 a filter bank shipped as an asset file).
 """
 import math
@@ -90,9 +93,10 @@ class S3TokenizerV2(nn.Module):
     """model_v2.py:354-415.  ``S3TokenizerV2(name, config)`` like the reference; ``config`` may be the reference's
     ``ModelConfig`` or anything with its attribute names (n_mels, n_audio_state, n_audio_head, n_audio_layer)."""
 
-    def __init__(self, name="speech_tokenizer_v2_25hz", config=None, weight_seed=None):
+    def __init__(self, name="speech_tokenizer_v2_25hz", config=None, weight_seed=None, precision="fp32"):
         super().__init__()
         self.name = name
+        self.precision = native.check_s3_precision(precision)
         g = lambda k, d: getattr(config, k, d) if config is not None else d
         self.n_mels, self.n_state = g("n_mels", 128), g("n_audio_state", 1280)
         self.n_head, self.n_layer = g("n_audio_head", 20), g("n_audio_layer", 6)
@@ -116,10 +120,11 @@ class S3TokenizerV2(nn.Module):
 
     def handle(self, device):
         device = torch.device(device)
-        if self._handle is None or self._handle.device != device:
+        native.check_s3_precision(self.precision)  # (the attribute may have been changed since)
+        if self._handle is None or self._handle.device != device or self._handle.precision != self.precision:
             sd = {k: v.detach().to(torch.float32).contiguous() for k, v in self.state_dict().items()}
             sd["rotary.cos"], sd["rotary.sin"] = precompute_rotary(64, 1024 * 2)  # model_v2.py:307
-            self._handle = native.S3Handle(sd, device)
+            self._handle = native.S3Handle(sd, device, self.precision)
         return self._handle
 
     @torch.inference_mode()
