@@ -158,6 +158,22 @@ int32_t ls_s3_code_frames(int32_t T);
 int32_t ls_s3_quantize(ls_s3* h, const float* mel, const int32_t* mel_len, int32_t* codes, int32_t* code_len, float* hidden,
                        int32_t B, int32_t T, void* stream);
 
+/* ---- log-mel front end of the S3 speech tokenizer: log_mel_spectrogram (speech/tools/S3Tokenizer/s3tokenizer/utils.py,
+ * the Whisper front end) for a right-padded batch of 16 kHz clips, each clip computed as if it were alone:
+ *   frames t = 0 .. audio_len[b]/160 - 1: samples t*160 - 200 + j, j < 400, reflected about the clip's own ends
+ *     (i < 0 -> -i, i >= len -> 2(len-1) - i: torch.stft center=True, whose last frame the reference drops);
+ *   power = |rDFT(hann_periodic(400) * frame)|^2 (201 bins), fp32 on the CUDA cores;
+ *   e = log10(max(filters @ power, 1e-10)); mel = (max(e, max over the clip's mels and frames of e - 8) + 4) / 4.
+ * audio [B,S] fp32, audio_len [B], filters [n_mels,201] fp32 (the reference's mel_filters.npz asset, key mel_<n_mels>;
+ * n_mels in [1, 128]) -> mel [B,n_mels,S/160] fp32 (NCT: the mel input of ls_s3_quantize; frames at or past mel_len[b]
+ * are zero), mel_len [B] = audio_len[b] / 160.  Samples at or past audio_len[b] are never read, so whatever the padding
+ * holds (NaN included) a clip's mel is bitwise the same as computing it alone.  Invalid lengths: a clip with
+ * audio_len[b] < 201 (reflect padding needs more than 200 samples) or > S gets mel_len[b] = 0 and an all-zero mel;
+ * nothing out of bounds is read.  Stateless, no allocation and no host synchronisation (capturable in a CUDA graph).
+ * B <= 65535.  All pointers are device pointers. */
+int32_t ls_s3_log_mel(const float* audio, const int32_t* audio_len, const float* filters, int32_t n_mels, float* mel,
+                      int32_t* mel_len, int32_t B, int64_t S, void* stream);
+
 /* ---- end to end with HOST buffers (pinned or pageable): H2D copies, solve, decode, D2H copy, and a
  * stream synchronise all happen inside the call.  wav_host: [B,1,T*hop]. */
 int32_t ls_synthesize_host(ls_flow* flow, ls_dac* dac, const float* mu_host, const float* mask_host,

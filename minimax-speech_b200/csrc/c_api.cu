@@ -460,6 +460,16 @@ int32_t ls_fsq_encode(const float* hidden, const float* project_down_weight, con
   });
 }
 
+int32_t ls_s3_log_mel(const float* audio, const int32_t* audio_len, const float* filters, int32_t n_mels, float* mel,
+                      int32_t* mel_len, int32_t B, int64_t S, void* stream) {
+  return ls::guarded([&] {
+    ls::require(audio && audio_len && filters && mel && mel_len, "ls_s3_log_mel: null argument");
+    ls::require(B > 0 && B <= 65535 && S >= 0, "ls_s3_log_mel: B must be in [1, 65535] and S >= 0");
+    ls::require(n_mels >= 1 && n_mels <= 128, "ls_s3_log_mel: n_mels must be in [1, 128]");
+    LS_CUDA(ls::launch_s3_log_mel(audio, audio_len, filters, n_mels, mel, mel_len, B, S, (cudaStream_t)stream));
+  });
+}
+
 int32_t ls_mask_to_lengths(const float* mask, int32_t* lengths, int32_t B, int32_t T, void* stream) {
   return ls::guarded([&] {
     ls::require(mask && lengths && B > 0 && T > 0, "ls_mask_to_lengths: bad argument");

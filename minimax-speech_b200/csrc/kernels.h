@@ -235,6 +235,11 @@ cudaError_t launch_groupnorm_mish(const float* x, float2* stats, const float* ga
 // FSQCodebook.encode of the S3 tokenizer: x fp32 [rows][D], w [8][D], bias [8] -> tokens int32 [rows] in [0, 3^8)
 cudaError_t launch_fsq_encode(const float* x, const float* w, const float* bias, int* tokens, long long rows, int D,
                               cudaStream_t s);
+// Log-mel front end of the S3 tokenizer (s3_mel.cu): right-padded audio fp32 [B][S] with audio_len [B], filters
+// [n_mels][201] (n_mels <= 128) -> mel fp32 [B][n_mels][S/160] (zeros past mel_len[b]), mel_len [B] = audio_len / 160,
+// or 0 (and an all-zero mel) when audio_len[b] < 201 or > S.  B <= 65535.
+cudaError_t launch_s3_log_mel(const float* audio, const int* audio_len, const float* filters, int n_mels, float* mel,
+                              int* mel_len, int B, long long S, cudaStream_t s);
 // timestep conditioning for nt time values: sinusoidal embedding -> MLP -> per-resnet projections
 struct TimeEmbedParams {
   const float* t;        // [nt] device, or nullptr: the values come from t_host (nt <= 64) inside the kernel parameters

@@ -18,7 +18,7 @@ EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create
            "ls_dac_encode_lengths",
            "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
-           "ls_s3_create", "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize",
+           "ls_s3_create", "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize", "ls_s3_log_mel",
            "ls_flow_destroy",
            "ls_flow_estimator_forward", "ls_flow_solve", "ls_dac_create", "ls_dac_destroy", "ls_dac_hop_length",
            "ls_dac_decode", "ls_synthesize_host", "ls_fsq_encode", "ls_mask_to_lengths", "ls_graph_create", "ls_graph_buffer",
@@ -121,6 +121,7 @@ def load():
         lib.ls_s3_destroy.restype = None
         lib.ls_s3_code_frames.argtypes = [i32]
         lib.ls_s3_quantize.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, vp]
+        lib.ls_s3_log_mel.argtypes = [vp, vp, vp, i32, vp, vp, i32, i64, vp]
         lib.ls_synthesize_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp, i32, f32, f32, vp, i32, i32, vp]
         lib.ls_mask_to_lengths.argtypes = [vp, vp, i32, i32, vp]
         lib.ls_fsq_encode.argtypes = [vp, vp, vp, vp, i64, i32, vp]
@@ -390,6 +391,18 @@ class DacHandle:
         check(load().ls_dac_decode(self._h, ptr(z), ptr(lengths), ptr(wav), B, L,
                                    current_stream_ptr(self.device)), "ls_dac_decode")
         return wav
+
+
+def s3_log_mel(audio, audio_len, filters):
+    """audio [B, S] float32, audio_len [B] int32, filters [n_mels, 201] float32 (all on one device, contiguous) ->
+    mel [B, n_mels, S // 160] float32 (zeros past each clip's frames), mel_len [B] int32 (ls_s3_log_mel)."""
+    B, S = audio.shape
+    n_mels = filters.shape[0]
+    mel = torch.empty(B, n_mels, S // 160, device=audio.device, dtype=torch.float32)
+    mel_len = torch.empty(B, device=audio.device, dtype=torch.int32)
+    check(load().ls_s3_log_mel(ptr(audio), ptr(audio_len), ptr(filters), n_mels, ptr(mel), ptr(mel_len), B, S,
+                               current_stream_ptr(audio.device)), "ls_s3_log_mel")
+    return mel, mel_len
 
 
 def mask_to_lengths(mask):

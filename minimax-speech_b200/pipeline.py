@@ -268,3 +268,48 @@ def extract_latents(paths, load_audio, encoder, device, rank=0, world_size=1, sa
         else:
             out.append((None, rec))
     return out
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Bulk token extraction: 16 kHz audio -> S3 tokenizer ids (the tokens the flow's input_embedding consumes)
+# ---------------------------------------------------------------------------------------------------------------------
+def token_record(tokens, n_samples, path, sample_rate=16000):
+    """The ``*_fsq.pt`` dict written by ``extract_tokens`` (CPU tensors).  This layout is this project's choice, modelled
+    on ``latent_record``; it has not been checked against what the reference's data loader reads."""
+    tokens = tokens.to(torch.int64).cpu()
+    return {"tokens": tokens, "token_len": int(tokens.shape[0]), "sample_rate": sample_rate,
+            "original_samples": n_samples, "original_path": path}
+
+
+def extract_tokens(paths, load_audio, tokenizer, device, rank=0, world_size=1, save=True, max_batch_samples=None):
+    """Tokenize this rank's share of ``paths`` (``shard_files``) with an ``S3TokenizerV2`` and write
+    ``<stem>_fsq.pt`` (``token_record``) next to each input.  ``load_audio(path) -> 1-D float tensor`` of 16 kHz mono
+    audio (decoding and resampling stay with the caller).
+
+    By default each file is one ``quantize_audio`` call.  ``max_batch_samples`` tokenizes length-sorted micro-batches of
+    at most that many padded samples (batch size x longest file, see ``plan_micro_batches``) in one call each, with
+    per-file lengths, so every file's mel is the one it gets alone; the share is loaded into host memory first.  Returns
+    the list of (output path or None, record) in file order."""
+    import os
+    start, end = shard_files(len(paths), rank, world_size)
+    mine = paths[start:end]
+    audio = [torch.as_tensor(load_audio(path), dtype=torch.float32).reshape(-1) for path in mine]
+    recs = [None] * len(mine)
+    for batch in plan_micro_batches([a.shape[0] for a in audio], max_batch_samples):
+        lens = [audio[i].shape[0] for i in batch]
+        buf = torch.zeros(len(batch), max(lens))
+        for b, i in enumerate(batch):
+            buf[b, :lens[b]] = audio[i]
+        codes, code_len = tokenizer.quantize_audio(buf.to(device), lens)
+        codes, code_len = codes.cpu(), code_len.tolist()
+        for b, i in enumerate(batch):  # (copies: a saved view would carry the whole batch's storage)
+            recs[i] = token_record(codes[b, :code_len[b]].clone(), lens[b], mine[i])
+    out = []
+    for path, rec in zip(mine, recs):
+        if save:
+            rec_path = os.path.splitext(path)[0] + "_fsq.pt"
+            torch.save(rec, rec_path)
+            out.append((rec_path, rec))
+        else:
+            out.append((None, rec))
+    return out
