@@ -127,6 +127,16 @@ int32_t ls_front_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_
 void ls_front_destroy(ls_front* h);
 int32_t ls_front_encode(ls_front* h, const int64_t* tokens, const float* embedding, float* mu, float* spks, int32_t B,
                         int32_t T, int32_t n_context, int32_t streaming, const int32_t* token_len, void* stream);
+/* Session mode: a batch of independent calls, e.g. one streaming hop of each of B sessions.  Row b of tokens [B,T_all]
+ * holds token_len[b] tokens (prompt tokens included), of which the last n_context[b] (0: finalize = True, 3: a
+ * non-final hop) are look-ahead context, and comes out equal to ls_front_encode of that row alone with its own
+ * n_context: T_b = token_len[b] - n_context[b] output tokens, mu [B,80,2T] with T = max T_b (the caller's), zero past
+ * 2 T_b.  The padding after a row's tokens is never read.  token_len, n_context: DEVICE int32 [B].  A row with
+ * n_context not 0 or 3, T_b < 1, token_len[b] > T_all or T_b > T gets an all-zero mu (no host synchronisation: the
+ * entries are only read on the device).  Needs T <= T_all; B <= 512 on the tensor-core path. */
+int32_t ls_front_encode_sessions(ls_front* h, const int64_t* tokens, const float* embedding, float* mu, float* spks, int32_t B,
+                                 int32_t T_all, int32_t T, const int32_t* token_len, const int32_t* n_context, int32_t streaming,
+                                 void* stream);
 
 /* ---- speaker encoder (SURVEY section 8 f-4): LearnableSpeakerEncoder.forward (speech/cosyvoice/llm/llm.py:34-96, blocks:
  * speech/cosyvoice/transformer/arch_util.py:21-123) and the averaging over several reference clips of

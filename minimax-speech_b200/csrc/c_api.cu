@@ -257,6 +257,17 @@ int32_t ls_front_encode(ls_front* h, const int64_t* tokens, const float* embeddi
                           token_len, (cudaStream_t)stream);
   });
 }
+int32_t ls_front_encode_sessions(ls_front* h, const int64_t* tokens, const float* embedding, float* mu, float* spks, int32_t B,
+                                 int32_t T_all, int32_t T, const int32_t* token_len, const int32_t* n_context, int32_t streaming,
+                                 void* stream) {
+  return ls::guarded([&] {
+    ls::require(h && tokens && embedding && mu && spks && token_len && n_context, "ls_front_encode_sessions: null argument");
+    ls::SerialScope scope(h->serial, h->device(), (cudaStream_t)stream);
+    const auto* tok = reinterpret_cast<const long long*>(tokens);
+    if (h->eng) h->eng->encode_sessions(tok, embedding, mu, spks, B, T_all, T, token_len, n_context, streaming != 0, (cudaStream_t)stream);
+    else h->eng32->encode_sessions(tok, embedding, mu, spks, B, T_all, T, token_len, n_context, streaming != 0, (cudaStream_t)stream);
+  });
+}
 
 int32_t ls_speaker_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_speaker** out) {
   return ls::guarded([&] {

@@ -362,11 +362,18 @@ __global__ void zero_tail_nct_kernel(float* __restrict__ y, const int* __restric
   if (i >= n) return;
   if ((int)(i % T) >= lens[i / ((size_t)C * T)]) y[i] = 0.f;
 }
-// lens0[b] = min(token_len[b], T) (keys at 25 Hz), lens1[b] = 2 * lens0[b] (keys and valid frames at 50 Hz)
-__global__ void front_lens_kernel(const int* __restrict__ token_len, int* __restrict__ lens0, int* __restrict__ lens1, int B, int T) {
+// lens0[b] = min(token_len[b], T) (keys at 25 Hz), lens1[b] = 2 * lens0[b] (keys and valid frames at 50 Hz).
+// Session mode (n_ctx != nullptr): lens0[b] = token_len[b] - n_ctx[b], the row's own output tokens, or 0 for a row
+// with invalid entries (its mu comes out all zero).
+__global__ void front_lens_kernel(const int* __restrict__ token_len, const int* __restrict__ n_ctx, int* __restrict__ lens0,
+                                  int* __restrict__ lens1, int B, int T_all, int T) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int l = max(0, min(token_len[b], T));
+  int l = max(0, min(token_len[b], T));
+  if (n_ctx) {
+    const int n = token_len[b], c = n_ctx[b];
+    l = ((c == 0 || c == 3) && n - c >= 1 && n <= T_all && n - c <= T) ? n - c : 0;
+  }
   lens0[b] = l, lens1[b] = 2 * l;
 }
 __global__ void scale_kernel(float* __restrict__ x, float sc, size_t n) {
@@ -1110,8 +1117,20 @@ float* FrontEngineF32::embed(const std::string& p, const float* x, int B, int T,
 // attention with chunk_ tokens at 25 Hz and 2*chunk_ frames at 50 Hz.
 void FrontEngineF32::encode(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all,
                             int n_context, bool streaming, const int* token_len, cudaStream_t s) {
-  const int T = T_all - n_context;
-  require(B > 0 && T > 0 && (n_context == 0 || n_context == 3), "B, T must be positive; context is 0 or 3 tokens");
+  require(B > 0 && T_all - n_context > 0 && (n_context == 0 || n_context == 3), "B, T must be positive; context is 0 or 3 tokens");
+  run(tokens, embedding, mu, spks, B, T_all, T_all - n_context, streaming, token_len, nullptr, s);
+}
+
+void FrontEngineF32::encode_sessions(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all,
+                                     int T, const int* token_len, const int* n_context, bool streaming, cudaStream_t s) {
+  require(B > 0 && T > 0 && T <= T_all && token_len && n_context, "B, T must be positive, T <= T_all, lengths given");
+  run(tokens, embedding, mu, spks, B, T_all, T, streaming, token_len, n_context, s);
+}
+
+// T_all token rows per utterance in, T output tokens (2T frames) out; T_all > T: the rows past T are look-ahead context.
+// n_context (session mode, with token_len): per-utterance context, see front_lens_kernel.
+void FrontEngineF32::run(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T,
+                         bool streaming, const int* token_len, const int* n_context, cudaStream_t s) {
   LS_CUDA(cudaSetDevice(device_));
   scratch_.reset();
   // speaker embedding: normalise, project (flow.py:463, 469)
@@ -1125,16 +1144,19 @@ void FrontEngineF32::encode(const long long* tokens, const float* embedding, flo
   if (token_len) {
     lens0 = reinterpret_cast<int*>(scratch_.get((size_t)2 * B + 8, s));
     lens1 = lens0 + B;
-    F32_LAUNCH(front_lens_kernel, (B + 127) / 128, 128, s, token_len, lens0, lens1, B, T_all - n_context);
+    F32_LAUNCH(front_lens_kernel, (B + 127) / 128, 128, s, token_len, n_context, lens0, lens1, B, T_all, T);
   }
   F32_LAUNCH(embed_tokens_kernel, blocks(n_all), 256, s, tokens, w_.ptr("input_embedding.weight"), x0, d_, T_all, vocab_, n_all,
              token_len);
   // embed (Linear, LayerNorm, scale) is position-independent: tokens and context go through it together
   float* pe_all = nullptr;
   float* xe = embed("encoder.embed", x0, B, T_all, &pe_all, s);
+  // session mode: the rows past a session's tokens are the zeros F.pad feeds the pre-lookahead layer of a call alone
+  // (the reference's padded batch embeds them instead: bias and LayerNorm make them non-zero)
+  if (n_context) F32_LAUNCH(zero_tail_nct_kernel, blocks(n_all), 256, s, xe, token_len, d_, T_all, n_all);
   float* x = xe;
   float* pe = pe_all;
-  if (n_context > 0) {
+  if (T_all > T) {
     x = scratch_.get(n, s);
     F32_LAUNCH(slice_time_kernel, blocks(n), 256, s, xe, x, T_all, T, n);
     pe = scratch_.get((size_t)(2 * T - 1) * d_, s);

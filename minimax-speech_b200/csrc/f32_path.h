@@ -107,11 +107,16 @@ class FrontEngineF32 {
   // token_len (device, nullable): per-utterance token counts of a right-padded batch
   void encode(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int n_context,
               bool streaming, const int* token_len, cudaStream_t s);
+  // session mode: see FrontEngine::encode_sessions
+  void encode_sessions(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T,
+                       const int* token_len, const int* n_context, bool streaming, cudaStream_t s);
   int out_dim() const { return out_; }
   int spk_dim() const { return spk_; }
   int device() const { return device_; }
 
  private:
+  void run(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T, bool streaming,
+           const int* token_len, const int* n_context, cudaStream_t s);
   float* layer(const std::string& p, float* x, const float* pe, int B, int T, int chunk, const int* lens, cudaStream_t s);
   float* embed(const std::string& p, const float* x, int B, int T, float** pe, cudaStream_t s);
   int device_ = 0, d_ = 512, vocab_ = 6561, out_ = 80, spk_ = 192, heads_ = 8, n_blocks_ = 0, n_up_ = 0, chunk_ = 25;

@@ -21,22 +21,40 @@ __global__ void __launch_bounds__(64) front_gather_kernel(const long long* __res
   if (lens && (int)(r % T_all) >= lens[r / T_all]) v = make_uint4(0u, 0u, 0u, 0u);
   reinterpret_cast<uint4*>(e + r * kD)[threadIdx.x] = v;
 }
-// lens0[b] = min(token_len[b], T) (keys at 25 Hz), lens1[b] = 2 * lens0[b] (keys and valid frames at 50 Hz)
-__global__ void front_lens_kernel(const int* __restrict__ token_len, int* __restrict__ lens0, int* __restrict__ lens1, int B, int T) {
+// lens0[b] = min(token_len[b], T) (keys at 25 Hz), lens1[b] = 2 * lens0[b] (keys and valid frames at 50 Hz).
+// Session mode (n_ctx != nullptr): lens0[b] = token_len[b] - n_ctx[b], the row's own output tokens, or 0 for a row
+// with invalid entries (its mu comes out all zero).
+__global__ void front_lens_kernel(const int* __restrict__ token_len, const int* __restrict__ n_ctx, int* __restrict__ lens0,
+                                  int* __restrict__ lens1, int B, int T_all, int T) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int l = max(0, min(token_len[b], T));
+  int l = max(0, min(token_len[b], T));
+  if (n_ctx) {
+    const int n = token_len[b], c = n_ctx[b];
+    l = ((c == 0 || c == 3) && n - c >= 1 && n <= T_all && n - c <= T) ? n - c : 0;
+  }
   lens0[b] = l, lens1[b] = 2 * l;
 }
 
 // LayerNorm over the 512 channels of a row (eps 1e-5), times `scale` (the rel-pos encoding's sqrt(d) input scale,
-// embedding.py:268): fp32 (optional) and bf16 outputs.  One warp per row, the row held in registers.
+// embedding.py:268): fp32 (optional) and bf16 outputs.  One warp per row, the row held in registers.  lens (nullable):
+// rows r with r % T >= lens[r / T] are written as zeros (right padding of a batch of sessions: what F.pad gives the
+// pre-lookahead convolution of a call alone).
 __global__ void __launch_bounds__(128) front_ln_rows_kernel(const float* __restrict__ x, const float* __restrict__ g,
                                                             const float* __restrict__ be, float scale, float* __restrict__ yf,
-                                                            __nv_bfloat16* __restrict__ yb, long long R) {
+                                                            __nv_bfloat16* __restrict__ yb, long long R,
+                                                            const int* __restrict__ lens, int T) {
   const long long r = (long long)blockIdx.x * 4 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (r >= R) return;
+  if (lens && (int)(r % T) >= lens[r / T]) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      if (yf) reinterpret_cast<float4*>(yf + r * kD)[i * 32 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
+      reinterpret_cast<uint2*>(yb + r * kD)[i * 32 + lane] = make_uint2(0u, 0u);
+    }
+    return;
+  }
   const float4* xr = reinterpret_cast<const float4*>(x + r * kD);
   float4 v[4];
   float sum = 0.f;
@@ -331,8 +349,21 @@ const FrontEngine::Plan& FrontEngine::plan_for(int B, int T_all, int T) {
 
 void FrontEngine::encode(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all,
                          int n_context, bool streaming, const int* token_len, cudaStream_t s) {
-  const int T = T_all - n_context, T2 = 2 * T;
-  require(B > 0 && T > 0 && (n_context == 0 || n_context == 3), "B, T must be positive; context is 0 or 3 tokens");
+  require(B > 0 && T_all - n_context > 0 && (n_context == 0 || n_context == 3), "B, T must be positive; context is 0 or 3 tokens");
+  run(tokens, embedding, mu, spks, B, T_all, T_all - n_context, streaming, token_len, nullptr, s);
+}
+
+void FrontEngine::encode_sessions(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all,
+                                  int T, const int* token_len, const int* n_context, bool streaming, cudaStream_t s) {
+  require(B > 0 && T > 0 && T <= T_all && token_len && n_context, "B, T must be positive, T <= T_all, lengths given");
+  run(tokens, embedding, mu, spks, B, T_all, T, streaming, token_len, n_context, s);
+}
+
+// T_all token rows per utterance in, T output tokens (2T frames) out; T_all > T: the rows past T are look-ahead context.
+// n_context (session mode, with token_len): per-utterance context, see front_lens_kernel.
+void FrontEngine::run(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T,
+                      bool streaming, const int* token_len, const int* n_context, cudaStream_t s) {
+  const int T2 = 2 * T;
   LS_CUDA(cudaSetDevice(device_));
   ensure_workspace(B, T_all, T, s);
   const Plan& pl = plan_for(B, T_all, T);
@@ -361,9 +392,10 @@ void FrontEngine::encode(const long long* tokens, const float* embedding, float*
     p.k_true = w.K, p.tag = 0, p.halo_mode = (halo && w.taps > 1) ? conv_halo_mode() : 0;
     LS_CUDA(launch_conv_gemm(a, a, w.map, p, num_sms_, s));
   };
-  auto ln = [&](const float* in, size_t g, size_t b, float scale, float* of, __nv_bfloat16* ob, long long R) {
+  auto ln = [&](const float* in, size_t g, size_t b, float scale, float* of, __nv_bfloat16* ob, long long R,
+                const int* zero_past = nullptr) {
     count_launch();
-    front_ln_rows_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(in, f32(g), f32(b), scale, of, ob, R);
+    front_ln_rows_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(in, f32(g), f32(b), scale, of, ob, R, zero_past, T_all);
     LS_CUDA(cudaGetLastError());
   };
   auto rel_pos = [&](int Tl) {
@@ -439,7 +471,7 @@ void FrontEngine::encode(const long long* tokens, const float* embedding, float*
     require(B <= 512, "at most 512 utterances per call with token lengths");
     lens0 = ws<int>(o_spk_), lens1 = lens0 + 512;
     count_launch();
-    front_lens_kernel<<<(B + 127) / 128, 128, 0, s>>>(token_len, lens0, lens1, B, T);
+    front_lens_kernel<<<(B + 127) / 128, 128, 0, s>>>(token_len, n_context, lens0, lens1, B, T_all, T);
     LS_CUDA(cudaGetLastError());
   }
   front_gather_kernel<<<(unsigned)((size_t)B * T_all), 64, 0, s>>>(tokens, arena_.ptr<__nv_bfloat16>(emb_table_), hb, vocab_, T_all,
@@ -450,14 +482,16 @@ void FrontEngine::encode(const long long* tokens, const float* embedding, float*
     ConvGemmParams p{};
     p.out0 = y, p.out0_dtype = OUT_F32;
     conv(pl.tok, embed_.lin, B, T_all, 0, p);
-    ln(y, embed_.g, embed_.b, sqrt_d, x, nb, (long long)B * T_all);
+    // session mode: the rows past a session's tokens are the zeros F.pad feeds the pre-lookahead layer of a call alone
+    // (the reference's padded batch embeds them instead: bias and LayerNorm make them non-zero)
+    ln(y, embed_.g, embed_.b, sqrt_d, x, nb, (long long)B * T_all, n_context ? token_len : nullptr);
   }
   float* xr = x;
   {  // PreLookaheadLayer (upsample_encoder.py:66-107): [x | context or zeros] -> conv k=4 -> leaky_relu -> causal conv k=3, + x
     ConvGemmParams p{};
     p.act = ACT_LRELU001, p.out1 = att, p.out1_mode = OUT1_COPY;
     conv(pl.pre1, pre1_, B, T, 0, p);  // reads rows t .. t+3 of the T_all-row input (rows past it are zero)
-    if (n_context > 0) {  // the residual stream keeps the first T rows of every utterance
+    if (T_all > T) {  // the residual stream keeps the first T rows of every utterance
       LS_CUDA(cudaMemcpy2DAsync(y, (size_t)T * kD * 4, x, (size_t)T_all * kD * 4, (size_t)T * kD * 4, B, cudaMemcpyDeviceToDevice, s));
       xr = y;
     }

@@ -23,11 +23,19 @@ class FrontEngine {
   // token_len (device, nullable): per-utterance token counts of a right-padded batch (mu is zero past 2 * token_len)
   void encode(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int n_context,
               bool streaming, const int* token_len, cudaStream_t s);
+  // Session mode: row b holds token_len[b] tokens of which the last n_context[b] (0 or 3) are look-ahead context, and
+  // comes out equal to an encode of that row alone: mu [B,80,2T], zero past 2 * (token_len[b] - n_context[b]).  Rows
+  // with invalid entries (n_context not 0 or 3, fewer than 1 output token, token_len > T_all or more than T output
+  // tokens) get an all-zero mu.  token_len and n_context are device int32 [B].
+  void encode_sessions(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T,
+                       const int* token_len, const int* n_context, bool streaming, cudaStream_t s);
   int out_dim() const { return out_; }
   int spk_dim() const { return spk_; }
   int device() const { return device_; }
 
  private:
+  void run(const long long* tokens, const float* embedding, float* mu, float* spks, int B, int T_all, int T, bool streaming,
+           const int* token_len, const int* n_context, cudaStream_t s);
   struct LayerW {
     PackedLinear qkv, pos, out, ff1, ff2;
     size_t g_mha, b_mha, g_ff, b_ff, bias_u, bias_v;

@@ -3,8 +3,10 @@ section 8 row f-1): speaker-embedding normalise + ``spk_embed_affine_layer``, ``
 ``UpsampleConformerEncoder`` (transformer/upsample_encoder.py) and ``encoder_proj``.  Parameters are registered under the
 reference's state_dict keys, so the flow checkpoint loads unchanged.  ``precision="bf16"`` (default): tensor-core path
 (csrc/front_engine.cu); ``"fp32"``: CUDA-core kernels of csrc/f32_path.cu.  Equal-length or right-padded batches; final chunks
-(finalize=True) and non-final chunks (3 look-ahead context tokens), optional block-causal streaming attention.  ``CausalMaskedDiffWithXvec`` is the drop-in for the reference's
-pipeline class: the same ``inference`` signature (prompt tokens, prompt latents, x-vector or reference mels)."""
+(finalize=True) and non-final chunks (3 look-ahead context tokens), optional block-causal streaming attention; ``encode_sessions``
+batches independent calls with a per-row look-ahead.  ``CausalMaskedDiffWithXvec`` is the drop-in for the reference's
+pipeline class: the same ``inference`` signature (prompt tokens, prompt latents, x-vector or reference mels), and
+``inference_batch`` for many utterances in one call."""
 import torch
 import torch.nn as nn
 
@@ -65,6 +67,31 @@ class TokenToMu(nn.Module):
                 raise NotImplementedError("right-padded batches of non-final chunks (the reference call is batch 1)")
             token_len = token_len.to(device=dev, dtype=torch.int32).contiguous()
         return self.handle(dev).encode(token.contiguous(), _as_f32(embedding, dev), n_ctx, streaming, token_len)
+
+    @torch.inference_mode()
+    def encode_sessions(self, token, token_len, n_context, embedding, streaming=False):
+        """A batch of independent calls in one launch sequence (e.g. one streaming hop of each of B sessions).
+        token [B,T_all] int64, right-padded; token_len [B]: tokens of each row, look-ahead included; n_context [B]: 0
+        (finalize=True) or 3 (the last 3 tokens are look-ahead context) per row; embedding [B,192].  Row b comes out
+        exactly as ``forward`` of that row alone with its own ``finalize``: -> (mu [B,80,2T], spks [B,80]) with
+        T = max(token_len - n_context), mu zero past ``2 * (token_len[b] - n_context[b])``.  The padding is never read."""
+        if token.dim() != 2 or token.shape[1] < 1 or token.dtype != torch.int64:
+            raise ValueError("token must be an int64 tensor [B, T_all >= 1]")
+        B, T_all = token.shape
+        if tuple(embedding.shape) != (B, self.spk_embed_dim):
+            raise ValueError(f"embedding must be [{B}, {self.spk_embed_dim}]")
+        n = torch.as_tensor(token_len).detach().cpu().reshape(-1)
+        c = torch.as_tensor(n_context).detach().cpu().reshape(-1)
+        if n.numel() != B or c.numel() != B or n.is_floating_point() or c.is_floating_point():
+            raise ValueError(f"token_len and n_context must be {B} integers each")
+        if bool(((c != 0) & (c != self.pre_lookahead_len)).any()):
+            raise ValueError(f"n_context must be 0 or {self.pre_lookahead_len} per row")
+        if bool(((n - c < 1) | (n > T_all)).any()):
+            raise ValueError(f"token_len must leave at least one token after the context and be at most {T_all}")
+        dev = token.device
+        i32 = lambda t: t.to(dtype=torch.int32).to(dev)  # noqa: E731
+        return self.handle(dev).encode_sessions(token.contiguous(), _as_f32(embedding, dev), int((n - c).max()), i32(n), i32(c),
+                                                streaming)
 
     @torch.inference_mode()
     def inference(self, token, embedding, decoder, n_timesteps=10, streaming=False, finalize=True):
@@ -169,6 +196,39 @@ class CausalMaskedDiffWithXvec(TokenToMu):
         mask = torch.ones(1, 1, mu.shape[2], device=dev)
         feat, _ = self.decoder(mu=mu, mask=mask, spks=spks, cond=cond, n_timesteps=10, streaming=streaming)
         return feat[:, :, mel_len1:].float(), None
+
+    @torch.inference_mode()
+    def inference_batch(self, token, prompt_token, prompt_feat, embedding, finalize, streaming=False):
+        """Padded-batch form of ``inference``: B independent utterances in one front call and one ``self.decoder`` call,
+        each equal to ``inference`` on it alone.  token, prompt_token: lists of B int tensors [1,T_b] / [1,Tp_b];
+        prompt_feat: list of B [1,Fp_b,80]; embedding [B,192]: each utterance's speaker embedding as
+        ``get_speaker_embedding`` returns it (used as is: normalising a unit vector again can change its last bits);
+        finalize: B bools (False: the last 3 tokens are look-ahead context).
+        -> (latents [B,80,max L] fp32, L [B] int64 on the host) with L_b = 2 (Tp_b + T_b [- 3]) - Fp_b; zero past L_b."""
+        B = len(token)
+        if B < 1 or not len(prompt_token) == len(prompt_feat) == len(finalize) == B:
+            raise ValueError("token, prompt_token, prompt_feat and finalize must hold one entry per utterance")
+        dev = embedding.device
+        rows = [torch.cat([p.reshape(-1).to(dev, torch.int64), t.reshape(-1).to(dev, torch.int64)]) for p, t in zip(prompt_token, token)]
+        n = torch.tensor([r.numel() for r in rows])
+        ctx = torch.tensor([0 if f else self.pre_lookahead_len for f in finalize])
+        mu, spks = self.encode_sessions(torch.nn.utils.rnn.pad_sequence(rows, batch_first=True), n, ctx, embedding, streaming)
+        frames = 2 * (n - ctx)
+        pf = torch.tensor([p.shape[1] for p in prompt_feat])
+        if bool((frames < pf).any()):
+            raise ValueError("prompt_feat is longer than the encoded token sequence")
+        T2 = mu.shape[2]
+        mask = (torch.arange(T2)[None, :] < frames[:, None]).float()[:, None, :].to(dev)
+        cond = torch.zeros_like(mu)
+        for b, p in enumerate(prompt_feat):
+            cond[b, :, :p.shape[1]] = _as_f32(p, dev)[0].transpose(0, 1)
+        feat, _ = self.decoder(mu=mu, mask=mask, spks=spks, cond=cond, n_timesteps=10, streaming=streaming)
+        # per-utterance cut at its prompt: frame Fp_b + t of row b -> frame t
+        L = frames - pf
+        t = torch.arange(int(L.max()))[None, :]
+        idx = (pf[:, None] + t).clamp(max=T2 - 1).to(dev)
+        out = feat.float().gather(2, idx[:, None, :].expand(B, feat.shape[1], -1))
+        return torch.where((t < L[:, None]).to(dev)[:, None, :], out, 0.0), L
 
     def forward(self, batch, device):
         raise NotImplementedError("training (flow.py:380-435) is out of scope; inference only")

@@ -16,7 +16,7 @@ OUT1_NONE, OUT1_LN, OUT1_COPY, OUT1_SNAKE = range(4)
 
 EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create", "ls_flow_create_fp16", "ls_flow_create_fp32", "ls_dac_create_fp32", "ls_dac_encode",
            "ls_dac_encode_lengths",
-           "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode",
+           "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode", "ls_front_encode_sessions",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
            "ls_s3_create", "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize", "ls_s3_log_mel",
            "ls_flow_destroy",
@@ -110,6 +110,7 @@ def load():
         lib.ls_front_destroy.argtypes = [vp]
         lib.ls_front_destroy.restype = None
         lib.ls_front_encode.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp]
+        lib.ls_front_encode_sessions.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, i32, vp]
         lib.ls_speaker_create.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_speaker_create_fp32.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_speaker_destroy.argtypes = [vp]
@@ -271,6 +272,16 @@ class FrontHandle:
         check(load().ls_front_encode(self._h, ptr(tokens), ptr(embedding), ptr(mu), ptr(spks), B, T, int(n_context),
                                      int(bool(streaming)), ptr(token_len) if token_len is not None else None,
                                      current_stream_ptr(self.device)), "ls_front_encode")
+        return mu, spks
+
+    def encode_sessions(self, tokens, embedding, T, token_len, n_context, streaming=False):
+        """Session mode (ls_front_encode_sessions): token_len / n_context are int32 device tensors [B]; mu [B,80,2T]."""
+        B, T_all = tokens.shape
+        mu = torch.empty(B, self.out_dim, 2 * T, device=tokens.device, dtype=torch.float32)
+        spks = torch.empty(B, self.out_dim, device=tokens.device, dtype=torch.float32)
+        check(load().ls_front_encode_sessions(self._h, ptr(tokens), ptr(embedding), ptr(mu), ptr(spks), B, T_all, int(T),
+                                              ptr(token_len), ptr(n_context), int(bool(streaming)),
+                                              current_stream_ptr(self.device)), "ls_front_encode_sessions")
         return mu, spks
 
 
