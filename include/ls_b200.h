@@ -242,7 +242,10 @@ int32_t ls_profile_end(ls_profile_entry* out, int32_t n_entries);
  * while it is set (NULL clears it).  Not used by any product path. */
 int32_t ls_debug_set_buffer(void* dev_ptr, int64_t bytes);
 
-/* ---- kernel-level hooks used by the parity tests (tests/test_kernels_gpu.py) ---- */
+/* ---- kernel-level hooks used by the kernel tests (tests/test_kernels_gpu.py, tests/test_kernel_plans_gpu.py) ----
+ * Test-only: not part of the product surface, no engine calls them.  num_sms: the SM count the launch plans for
+ * (0 = the device's own; a value outside [0, device SMs] is refused with LS_ERR_INVALID), so that small shapes reach
+ * the plans a full-size launch takes.  plan_out (may be NULL) receives the plan the launch used. */
 typedef struct ls_conv_gemm_desc {
   const void* a0; /* bf16 [B][T_in][a0_C] */
   const void* a1; /* optional second K source (channel concat), bf16 [B][T_in][a1_C] */
@@ -259,9 +262,9 @@ typedef struct ls_conv_gemm_desc {
   const float* temb;
   int64_t temb_bstride;
   const void* addend;
-  int32_t addend_dtype; /* 1 f32, 2 bf16 */
+  int32_t addend_dtype; /* 1 f32, 2 bf16, 3 fp16 */
   void* out0;
-  int32_t out0_dtype; /* 0 none, 1 f32, 2 bf16 */
+  int32_t out0_dtype; /* 0 none, 1 f32, 2 bf16, 3 fp16 */
   void* out1;
   int32_t out1_mode; /* 0 none, 1 layernorm, 2 copy, 3 snake */
   const float* p1_a;
@@ -269,17 +272,20 @@ typedef struct ls_conv_gemm_desc {
   int32_t n_store;
   int64_t out_ld, out_shift, out_bstride, out_alloc, out_valid_mul;
 } ls_conv_gemm_desc;
-int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, void* stream);
+/* plan_out: int32[8] = grid, the largest tile count of any CTA, dual issue, resident weights, activation stages,
+ * weight stages, TMA stores, halo mode (all 0 when there is nothing to launch) */
+int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* plan_out, void* stream);
 /* qkv bf16 [B][T][3*H*64] -> out bf16 [B][T][H*64] */
 int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, int32_t B, int32_t T, int32_t H,
                           int32_t chunk, void* stream);
 
 /* Fused transformer-block tail (tblock.cu): att bf16 [R][512], u fp32 [R][256] (updated in place when
  * tail_mode == 0), bf16 weights wo [256][512], w1 [1024][256], w2 [256][1024], wqkv [1536][256], vec = 2560 floats
- * (bo, g3, be3, b1, b2, g1n, be1n).  tail_mode 0 -> qkv_out bf16 [R][1536]; 1 -> tail_out bf16 [R][256]. */
+ * (bo, g3, be3, b1, b2, g1n, be1n).  tail_mode 0 -> qkv_out bf16 [R][1536]; 1 -> tail_out bf16 [R][256].
+ * plan_out: int32[2] = grid, the largest tile count of any CTA. */
 int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1, const void* w2, const void* wqkv,
                        const float* vec, void* qkv_out, void* tail_out, const int32_t* lengths, int32_t R, int32_t T,
-                       int32_t tail_mode, void* stream);
+                       int32_t tail_mode, int32_t num_sms, int32_t* plan_out, void* stream);
 
 #ifdef __cplusplus
 }

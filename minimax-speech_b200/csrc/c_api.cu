@@ -557,6 +557,17 @@ struct ls_graph {
   }
 };
 
+namespace {
+// the SM count a test hook launches for: 0 = the device's own; anything outside [0, device SMs] is refused
+int test_hook_sms(int32_t num_sms, const char* what) {
+  int dev = 0, sms = 0;
+  LS_CUDA(cudaGetDevice(&dev));
+  LS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  ls::require(num_sms >= 0 && num_sms <= sms, std::string(what) + ": num_sms outside [0, device SMs]");
+  return num_sms == 0 ? sms : num_sms;
+}
+}  // namespace
+
 extern "C" {
 
 int32_t ls_graph_create(ls_flow* flow, ls_dac* dac, const float* noise_dev, int64_t noise_stride, const float* t_span_host,
@@ -650,12 +661,10 @@ int32_t ls_profile_end(ls_profile_entry* out4, int32_t n_entries) {
   });
 }
 
-int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, void* stream) {
+int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* plan_out, void* stream) {
   return ls::guarded([&] {
     ls::require(d && d->a0 && d->w, "ls_test_conv_gemm: null argument");
-    int dev = 0, sms = 0;
-    LS_CUDA(cudaGetDevice(&dev));
-    LS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int sms = test_hook_sms(num_sms, "ls_test_conv_gemm");
     CUtensorMap a0, a1, w;
     const bool halo = ls::conv_halo_enabled();
     const int box = halo ? ls::conv_halo_box_rows(d->taps, d->dil) : 128;
@@ -679,7 +688,7 @@ int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, void* stream) {
     p.out_ld = d->out_ld, p.out_shift = d->out_shift, p.out_bstride = d->out_bstride, p.out_alloc = d->out_alloc;
     p.out_valid_mul = d->out_valid_mul;
     p.k_true = d->K, p.tag = 0, p.halo_mode = ls::conv_halo_mode();
-    LS_CUDA(ls::launch_conv_gemm(a0, a1, w, p, sms, (cudaStream_t)stream));
+    LS_CUDA(ls::launch_conv_gemm(a0, a1, w, p, sms, (cudaStream_t)stream, plan_out));
   });
 }
 
@@ -700,12 +709,10 @@ int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, in
 
 int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1, const void* w2, const void* wqkv,
                        const float* vec, void* qkv_out, void* tail_out, const int32_t* lengths, int32_t R, int32_t T,
-                       int32_t tail_mode, void* stream) {
+                       int32_t tail_mode, int32_t num_sms, int32_t* plan_out, void* stream) {
   return ls::guarded([&] {
     ls::require(att && u && wo && w1 && w2 && wqkv && vec, "ls_test_tblock: null argument");
-    int dev = 0, sms = 0;
-    LS_CUDA(cudaGetDevice(&dev));
-    LS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const int sms = test_hook_sms(num_sms, "ls_test_tblock");
     ls::require(tail_mode != 1 ? qkv_out != nullptr : tail_out != nullptr, "ls_test_tblock: missing output");
     ls::TBlockMaps m;
     ls::require(ls::make_tile_map(&m.att, att, 2, 512, R, 128) && ls::make_tile_map(&m.u, u, 4, 256, R, 128),
@@ -724,7 +731,7 @@ int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1
       ls::require(ls::make_tile_map(&m.tail_out, tail_out, 2, 256, R, 128), "tensor map tail", LS_ERR_CUDA);
     ls::TBlockParams p{};
     p.R = R, p.T = T, p.lengths = lengths, p.vec = vec, p.tail_mode = tail_mode;
-    LS_CUDA(ls::launch_tblock(m, p, sms, (cudaStream_t)stream));
+    LS_CUDA(ls::launch_tblock(m, p, sms, (cudaStream_t)stream, plan_out));
   });
 }
 

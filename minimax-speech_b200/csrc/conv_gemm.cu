@@ -1171,10 +1171,13 @@ cudaError_t launch_instance(int grid, size_t smem, cudaStream_t stream, const CU
 }  // namespace
 
 cudaError_t LS_FN(launch_conv_gemm)(const CUtensorMap& mapA0, const CUtensorMap& mapA1, const CUtensorMap& mapW,
-                                    const ConvGemmParams& p, int num_sms, cudaStream_t stream) {
+                                    const ConvGemmParams& p, int num_sms, cudaStream_t stream, int* plan_out) {
 #if !LS_HALF_FP16
-  if (p.fp16) return launch_conv_gemm_fp16(mapA0, mapA1, mapW, p, num_sms, stream);  // fp16-operand build of this file
+  if (p.fp16) return launch_conv_gemm_fp16(mapA0, mapA1, mapW, p, num_sms, stream, plan_out);  // fp16-operand build of this file
 #endif
+  if (plan_out)
+    for (int i = 0; i < kConvPlanInts; ++i) plan_out[i] = 0;
+  if (num_sms <= 0) return cudaErrorInvalidValue;
   if (p.block_n % 16 || p.block_n < 16 || p.block_n > 256 || p.N % p.block_n || p.chan_mod % 16) return cudaErrorInvalidValue;
   if ((p.act == ACT_LN_MISH || p.out1_mode == OUT1_LN) && p.block_n != p.N) return cudaErrorInvalidValue;
   if (p.out1_mode == OUT1_LN && p.out0_dtype != OUT_F32) return cudaErrorInvalidValue;
@@ -1293,6 +1296,11 @@ cudaError_t LS_FN(launch_conv_gemm)(const CUtensorMap& mapA0, const CUtensorMap&
   }
   const CUtensorMap* mo0 = &mo0v;
   const CUtensorMap* mo1 = &mo1v;
+  if (plan_out) {
+    const int plan[kConvPlanInts] = {grid, (int)((total + grid - 1) / grid), pp.dual, pp.b_resident, pp.a_stages,
+                                     pp.b_stages, pp.tma_out, pp.halo_mode};
+    for (int i = 0; i < kConvPlanInts; ++i) plan_out[i] = plan[i];
+  }
   const int add = p.addend_dtype == ADD_GEMM ? (int)ADD_GEMM : p.addend ? p.addend_dtype : (int)OUT_NONE;
   const int temb = p.temb ? 1 : 0;
 #define LS_CONV_CASE(A, O0, O1, AD, TE)                                                                          \

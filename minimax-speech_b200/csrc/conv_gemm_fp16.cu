@@ -5,7 +5,7 @@
 #else  // development aid: a library without the fp16-operand kernels
 #include "kernels.h"
 namespace ls {
-cudaError_t launch_conv_gemm_fp16(const CUtensorMap&, const CUtensorMap&, const CUtensorMap&, const ConvGemmParams&, int, cudaStream_t) {
+cudaError_t launch_conv_gemm_fp16(const CUtensorMap&, const CUtensorMap&, const CUtensorMap&, const ConvGemmParams&, int, cudaStream_t, int*) {
   return cudaErrorNotSupported;
 }
 }  // namespace ls

@@ -135,11 +135,15 @@ struct ConvGemmParams {
 inline int conv_halo_box_rows(int taps, int dil) { return 128 + (taps - 1) * dil; }
 __host__ __device__ constexpr int ls_conv_a_stage_bytes(int box_rows) { return ((box_rows + 7) / 8) * 1024; }
 
-// Tensor maps are created on the host (tma_host.cpp helpers) and passed by value.
+// Tensor maps are created on the host (tma_host.cpp helpers) and passed by value.  The grid is at most num_sms CTAs.
+// plan_out (optional, the kernel tests' hook): receives the plan the launch used, kConvPlanInts values:
+// grid, the largest tile count of any CTA, dual, b_resident, a_stages, b_stages, tma_out, halo_mode (all 0 when there
+// is nothing to launch).
+constexpr int kConvPlanInts = 8;
 cudaError_t launch_conv_gemm(const CUtensorMap& mapA0, const CUtensorMap& mapA1, const CUtensorMap& mapW,
-                             const ConvGemmParams& p, int num_sms, cudaStream_t stream);
+                             const ConvGemmParams& p, int num_sms, cudaStream_t stream, int* plan_out = nullptr);
 cudaError_t launch_conv_gemm_fp16(const CUtensorMap& mapA0, const CUtensorMap& mapA1, const CUtensorMap& mapW,
-                                  const ConvGemmParams& p, int num_sms, cudaStream_t stream);
+                                  const ConvGemmParams& p, int num_sms, cudaStream_t stream, int* plan_out = nullptr);
 
 // Flash attention forward over a packed [B][T][3*H*64] bf16 QKV tensor (Q | K | V column blocks).
 #ifndef ATTN_KV
@@ -200,8 +204,12 @@ struct TBlockMaps {
   CUtensorMap qkv_out;   // bf16 [R][1536] next block's Q | K | V          (box 64 x 128)   tail_mode 0
   CUtensorMap tail_out;  // bf16 [R][256]  u'' masked                      (box 64 x 128)   tail_mode 1
 };
-cudaError_t launch_tblock(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream);
-cudaError_t launch_tblock_fp16(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream);
+// The grid is at most num_sms CTAs (fewer when clusters do not all fit at once).  plan_out (optional, the kernel tests'
+// hook): receives the grid and the largest tile count of any CTA.
+cudaError_t launch_tblock(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream,
+                          int* plan_out = nullptr);
+cudaError_t launch_tblock_fp16(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream,
+                               int* plan_out = nullptr);
 
 // ---- bandwidth kernels (elementwise.cu) ----
 // NCT fp32 [B][C][T] -> time-major bf16 dst[b][t][c_off + c], dst row stride ld; rows >= len zeroed.

@@ -1152,31 +1152,42 @@ tblock_kernel(const __grid_constant__ CUtensorMap mapAtt, const __grid_constant_
 
 }  // namespace
 
-cudaError_t LS_FN(launch_tblock)(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream) {
+cudaError_t LS_FN(launch_tblock)(const TBlockMaps& m, const TBlockParams& p, int num_sms, cudaStream_t stream,
+                                 int* plan_out) {
 #if !LS_HALF_FP16
-  if (p.fp16) return launch_tblock_fp16(m, p, num_sms, stream);  // fp16-operand build of this file
+  if (p.fp16) return launch_tblock_fp16(m, p, num_sms, stream, plan_out);  // fp16-operand build of this file
 #endif
-  if (p.R <= 0 || p.T <= 0 || p.vec == nullptr) return cudaErrorInvalidValue;
+  if (p.R <= 0 || p.T <= 0 || p.vec == nullptr || num_sms < kCS) return cudaErrorInvalidValue;
   static std::atomic<unsigned long long> optin{0};  // one bit per device
   if (cudaError_t e = smem_optin_once(optin, reinterpret_cast<const void*>(tblock_kernel), kSmemBytes); e != cudaSuccess) return e;
   const int n_tiles = (p.R + kTileM - 1) / kTileM;
   const int n_groups = (n_tiles + kCS - 1) / kCS;
-  static int max_clusters = 0;
-  if (max_clusters == 0) {
-    max_clusters = num_sms / kCS;
-    if (kCS > 1) {  // clusters are placed inside one GPC: ask how many fit at once
+  int max_clusters = num_sms / kCS;
+  if (kCS > 1) {
+    // clusters are placed inside one GPC: ask how many fit at once.  The answer depends on the device only, so it is
+    // asked once per device (racing first calls may both ask; they get the same answer).
+    static std::atomic<int> fit[64];  // clusters of this kernel that fit at once, per device (0: not asked yet)
+    int dev = 0;
+    if (cudaError_t e = cudaGetDevice(&dev); e != cudaSuccess) return e;
+    int n = fit[dev & 63].load(std::memory_order_acquire);
+    if (n == 0) {
       cudaLaunchConfig_t qc = {};
       qc.gridDim = dim3(num_sms / kCS * kCS), qc.blockDim = dim3(kThreads), qc.dynamicSmemBytes = kSmemBytes;
       cudaLaunchAttribute qa[1];
       qa[0].id = cudaLaunchAttributeClusterDimension;
       qa[0].val.clusterDim.x = kCS, qa[0].val.clusterDim.y = 1, qa[0].val.clusterDim.z = 1;
       qc.attrs = qa, qc.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, tblock_kernel, &qc) == cudaSuccess && n > 0 && n < max_clusters)
-        max_clusters = n;
+      if (cudaOccupancyMaxActiveClusters(&n, tblock_kernel, &qc) != cudaSuccess || n < 0) n = 0;
+      if (n > 0) fit[dev & 63].store(n, std::memory_order_release);
     }
+    if (n > 0 && n < max_clusters) max_clusters = n;
   }
   const int grid = (n_groups < max_clusters ? n_groups : max_clusters) * kCS;
+  if (plan_out) {
+    const int ctas_groups = grid / kCS;
+    plan_out[0] = grid;
+    plan_out[1] = (n_groups + ctas_groups - 1) / ctas_groups;
+  }
   const double rows = (double)p.R;
   const double macs = (p.tail_mode == 2 ? 0.0 : (double)kInner * kC + 2.0 * kC * kFF) + (p.tail_mode != 1 ? (double)kC * kQKV : 0.0);
   const double bytes = (p.tail_mode == 2 ? rows * (kC * 4.0 + kQKV * 2.0)

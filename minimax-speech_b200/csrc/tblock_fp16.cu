@@ -5,6 +5,6 @@
 #else  // development aid: a library without the fp16-operand kernels
 #include "kernels.h"
 namespace ls {
-cudaError_t launch_tblock_fp16(const TBlockMaps&, const TBlockParams&, int, cudaStream_t) { return cudaErrorNotSupported; }
+cudaError_t launch_tblock_fp16(const TBlockMaps&, const TBlockParams&, int, cudaStream_t, int*) { return cudaErrorNotSupported; }
 }  // namespace ls
 #endif

@@ -136,15 +136,28 @@ def load():
         lib.ls_graph_destroy.restype = None
         lib.ls_debug_set_buffer.argtypes = [vp, i64]
         lib.ls_profile_end.argtypes = [C.POINTER(ProfileEntry), i32]
-        lib.ls_test_tblock.argtypes = [vp] * 10 + [i32, i32, i32, vp]
-        lib.ls_test_conv_gemm.argtypes = [C.POINTER(ConvGemmDesc), vp]
+        lib.ls_test_tblock.argtypes = [vp] * 10 + [i32, i32, i32, i32, vp, vp]
+        lib.ls_test_conv_gemm.argtypes = [C.POINTER(ConvGemmDesc), i32, vp, vp]
         lib.ls_test_attention.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
         for name in EXPORTS:
             fn = getattr(lib, name)
             if fn.restype is C.c_int:
                 fn.restype = i32
+        # the kernel test hooks' SM count and plan arguments (just before the stream) are optional for Python callers
+        lib.ls_test_conv_gemm = _plan_args_optional(lib.ls_test_conv_gemm, 1)
+        lib.ls_test_tblock = _plan_args_optional(lib.ls_test_tblock, 13)
         _lib = lib
         return lib
+
+
+def _plan_args_optional(fn, n_fixed):
+    """fn(fixed..., num_sms, plan_out, stream) also callable as fn(fixed..., stream): the device's SM count, no plan"""
+    def call(*args):
+        if len(args) == n_fixed + 1:
+            args = args[:-1] + (0, None, args[-1])
+        return fn(*args)
+    call.__name__ = fn.__name__
+    return call
 
 
 def check(code, what):

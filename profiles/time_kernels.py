@@ -40,7 +40,7 @@ def tblock(R, tail_mode=0):
     def fn():
         native.check(lib.ls_test_tblock(native.ptr(att), native.ptr(u), native.ptr(wo), native.ptr(w1), native.ptr(w2),
                                         native.ptr(wq), native.ptr(vec), native.ptr(qkv), native.ptr(tail), None, R, R,
-                                        tail_mode, s), "tblock")
+                                        tail_mode, 0, None, s), "tblock")
     us = timeit(fn)
     macs = (0 if tail_mode == 2 else 512 * 256 + 2 * 256 * 1024) + (256 * 1536 if tail_mode != 1 else 0)
     print(f"tblock R={R} tail={tail_mode}: {us:8.1f} us  {2.0 * R * macs / us / 1e6:7.1f} TFLOP/s")
