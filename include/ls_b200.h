@@ -184,6 +184,45 @@ int32_t ls_s3_quantize(ls_s3* h, const float* mel, const int32_t* mel_len, int32
 int32_t ls_s3_log_mel(const float* audio, const int32_t* audio_len, const float* filters, int32_t n_mels, float* mel,
                       int32_t* mel_len, int32_t B, int64_t S, void* stream);
 
+/* ---- sample-rate conversion: torchaudio.functional.resample(x, orig_freq, new_freq) at its defaults (sinc_interp_hann,
+ * lowpass_filter_width 6, rolloff 0.99; the resampler of the S3 tokenizer's load_audio and CosyVoice's front end) for a
+ * right-padded batch of clips, each converted as if it were alone.  With the ratio reduced to O / N (gcd), base =
+ * min(O, N) * 0.99 and width = ceil(6 O / base), output sample j = q*N + p of a clip is
+ *   sum_i x[q*O + i] k_p(i),  k_p(i) = sinc(pi t) cos^2(pi t / 12) base / O,  t = base (i/O - p/N),
+ * with x zero outside the clip; torchaudio sums i over [-width, width + O) with t clamped to +-6, this library only the
+ * taps with |t| < 6 (the others are below 1e-45).  The taps are computed once on the host in double and rounded once to
+ * fp32; each output sums its taps in increasing i in fp32.  Output length ceil(N len / O).  orig == new is a copy.
+ *
+ * ls_resampler_create builds the table for one (orig, new) pair and uploads it to `device` (LS_ERR_UNSUPPORTED for a
+ * table over 96 KiB, e.g. rates whose reduced ratio has thousands of phases); the handle is reused for any number of
+ * calls, which copy nothing.  ls_resample: audio [B,S_in] fp32 with audio_len [B] -> out [B,S_out] fp32, out_len [B] =
+ * ceil(N audio_len[b] / O); S_out >= ceil(N S_in / O) (the caller may pick a larger S_out, e.g. a multiple of a hop);
+ * out is zero from out_len[b] to S_out.  Samples at or past audio_len[b] are never read, so whatever the padding holds a
+ * clip's output is bitwise the same as converting it alone.  A length < 1 or > S_in gives out_len 0 and a zero row.
+ * B <= 65535, S_in and S_out < 2^31.  No allocation and no host synchronisation (capturable in a CUDA graph); the calls
+ * hold no per-call state, so one handle may serve several streams at once.  All pointers are device pointers.
+ * ls_resample_taps (host only, no device needed): the reduced ratio, torchaudio's width, the largest tap count of a phase,
+ * and (when the arrays are not NULL) the table ls_resample uses: first [N] (the first i of phase p), count [N], taps
+ * [N][max_taps] (zero-padded).  NULL arrays: sizes only.  LS_ERR_UNSUPPORTED (sizes other than max_taps still written)
+ * for a table over 96 KiB. */
+typedef struct ls_resampler ls_resampler;
+int32_t ls_resampler_create(int32_t orig_freq, int32_t new_freq, int32_t device, ls_resampler** out);
+void ls_resampler_destroy(ls_resampler* h);
+int32_t ls_resample(ls_resampler* h, const float* audio, const int32_t* audio_len, float* out, int32_t* out_len, int32_t B,
+                    int64_t S_in, int64_t S_out, void* stream);
+int32_t ls_resample_taps(int32_t orig_freq, int32_t new_freq, int32_t* orig_red, int32_t* new_red, int32_t* width,
+                         int32_t* max_taps, int32_t* first, int32_t* count, float* taps);
+
+/* ---- latent speed change: CosyVoice2's token2wav(speed) F.interpolate(feat, size=int(L / speed), mode='linear') on a
+ * right-padded batch of DAC latents.  z [B,C,L_in] -> out [B,C,L_out]: row b's first len_in[b] frames go to len_out[b]
+ * frames with PyTorch's align_corners=False arithmetic (scale = len_in / len_out, src = max(scale (d + 0.5) - 0.5, 0),
+ * i0 = (int)src, i1 = min(i0 + 1, len_in - 1), lambda = src - i0, out = (1 - lambda) x[i0] + lambda x[i1]), evaluated in
+ * double and rounded once to fp32 (= F.interpolate in float64, rounded); zero from len_out[b] to L_out.  len_in, len_out:
+ * DEVICE int32 [B] (the caller computes len_out, e.g. int(L / speed) in Python).  A row with len_in outside [1, L_in] or
+ * len_out outside [1, L_out] is all zero.  Stateless; all pointers are device pointers. */
+int32_t ls_latent_resize_linear(const float* z, const int32_t* len_in, const int32_t* len_out, float* out, int32_t B, int32_t C,
+                                int32_t L_in, int32_t L_out, void* stream);
+
 /* ---- end to end with HOST buffers (pinned or pageable): H2D copies, solve, decode, D2H copy, and a
  * stream synchronise all happen inside the call.  wav_host: [B,1,T*hop]. */
 int32_t ls_synthesize_host(ls_flow* flow, ls_dac* dac, const float* mu_host, const float* mask_host,

@@ -1,4 +1,5 @@
 // extern "C" surface declared in include/ls_b200.h.
+#include <algorithm>
 #include <atomic>
 #include <cstdarg>
 #include <mutex>
@@ -189,6 +190,17 @@ struct ls_s3 {
   int device() const { return eng ? eng->device() : eng32->device(); }
   std::unique_ptr<ls::S3Engine> eng;       // bf16x3 tensor-core mode (fp32-level error: tokens are rounding decisions)
   std::unique_ptr<ls::S3EngineF32> eng32;  // fp32 mode
+};
+
+struct ls_resampler {
+  int device = 0;
+  ls::ResamplePlan plan;
+  float* taps = nullptr;
+  int2* fc = nullptr;
+  ~ls_resampler() {
+    if (taps) cudaFree(taps);
+    if (fc) cudaFree(fc);
+  }
 };
 
 extern "C" {
@@ -478,6 +490,76 @@ int32_t ls_s3_log_mel(const float* audio, const int32_t* audio_len, const float*
     ls::require(B > 0 && B <= 65535 && S >= 0, "ls_s3_log_mel: B must be in [1, 65535] and S >= 0");
     ls::require(n_mels >= 1 && n_mels <= 128, "ls_s3_log_mel: n_mels must be in [1, 128]");
     LS_CUDA(ls::launch_s3_log_mel(audio, audio_len, filters, n_mels, mel, mel_len, B, S, (cudaStream_t)stream));
+  });
+}
+
+int32_t ls_resample_taps(int32_t orig_freq, int32_t new_freq, int32_t* orig_red, int32_t* new_red, int32_t* width,
+                         int32_t* max_taps, int32_t* first, int32_t* count, float* taps) {
+  return ls::guarded([&] {
+    ls::ResampleTable t;
+    const bool fill = first || count || taps;
+    const int code = ls::resample_table(orig_freq, new_freq, &t, fill);
+    if (orig_red) *orig_red = t.O;
+    if (new_red) *new_red = t.N;
+    if (width) *width = t.width;
+    if (max_taps) *max_taps = code == LS_OK ? t.max_taps : 0;
+    ls::require(code != LS_ERR_INVALID, "ls_resample_taps: rates must be positive");
+    ls::require(code == LS_OK, "ls_resample_taps: the tap table exceeds 96 KiB", LS_ERR_UNSUPPORTED);
+    if (first) std::copy(t.first.begin(), t.first.end(), first);
+    if (count) std::copy(t.count.begin(), t.count.end(), count);
+    if (taps) std::copy(t.taps.begin(), t.taps.end(), taps);
+  });
+}
+
+int32_t ls_resampler_create(int32_t orig_freq, int32_t new_freq, int32_t device, ls_resampler** out) {
+  return ls::guarded([&] {
+    ls::require(out != nullptr, "ls_resampler_create: null argument");
+    ls::ResampleTable t;
+    const int code = ls::resample_table(orig_freq, new_freq, &t);
+    ls::require(code != LS_ERR_INVALID, "ls_resampler_create: rates must be positive");
+    ls::require(code == LS_OK, "ls_resampler_create: the tap table exceeds 96 KiB", LS_ERR_UNSUPPORTED);
+    auto h = std::make_unique<ls_resampler>();
+    ls::require(ls::resample_plan(t, &h->plan) == LS_OK, "ls_resampler_create: the tile does not fit shared memory",
+                LS_ERR_UNSUPPORTED);
+    // device layout: rows padded to the plan's odd stride
+    const int N = t.N, stride = h->plan.stride;
+    std::vector<float> taps((size_t)N * stride, 0.0f);
+    std::vector<int2> fc(N);
+    for (int p = 0; p < N; ++p) {
+      std::copy_n(t.taps.begin() + (size_t)p * t.max_taps, t.max_taps, taps.begin() + (size_t)p * stride);
+      fc[p] = make_int2(t.first[p], t.count[p]);
+    }
+    h->device = device;
+    LS_CUDA(cudaSetDevice(device));
+    LS_CUDA(cudaMalloc(&h->taps, taps.size() * sizeof(float)));
+    LS_CUDA(cudaMalloc(&h->fc, fc.size() * sizeof(int2)));
+    LS_CUDA(cudaMemcpy(h->taps, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice));
+    LS_CUDA(cudaMemcpy(h->fc, fc.data(), fc.size() * sizeof(int2), cudaMemcpyHostToDevice));
+    h->plan.taps = h->taps, h->plan.fc = h->fc;
+    *out = h.release();
+  });
+}
+void ls_resampler_destroy(ls_resampler* h) { delete h; }
+int32_t ls_resample(ls_resampler* h, const float* audio, const int32_t* audio_len, float* out, int32_t* out_len, int32_t B,
+                    int64_t S_in, int64_t S_out, void* stream) {
+  return ls::guarded([&] {
+    ls::require(h && audio && audio_len && out && out_len, "ls_resample: null argument");
+    ls::require(B > 0 && B <= 65535 && S_in >= 1 && S_in <= INT32_MAX && S_out <= INT32_MAX,
+                "ls_resample: B must be in [1, 65535] and 1 <= S_in, S_out < 2^31");
+    const long long need = ((long long)h->plan.N * S_in + h->plan.O - 1) / h->plan.O;
+    ls::require(S_out >= need, "ls_resample: S_out must be at least ceil(new * S_in / orig) = " + std::to_string(need));
+    LS_CUDA(cudaSetDevice(h->device));
+    LS_CUDA(ls::launch_resample(h->plan, audio, audio_len, out, out_len, B, S_in, S_out, (cudaStream_t)stream));
+  });
+}
+
+int32_t ls_latent_resize_linear(const float* z, const int32_t* len_in, const int32_t* len_out, float* out, int32_t B, int32_t C,
+                                int32_t L_in, int32_t L_out, void* stream) {
+  return ls::guarded([&] {
+    ls::require(z && len_in && len_out && out, "ls_latent_resize_linear: null argument");
+    ls::require(B > 0 && C > 0 && L_in > 0 && L_out > 0 && (long long)B * C <= INT32_MAX,
+                "ls_latent_resize_linear: B, C, L_in, L_out must be positive");
+    LS_CUDA(ls::launch_latent_resize_linear(z, len_in, len_out, out, B, C, L_in, L_out, (cudaStream_t)stream));
   });
 }
 

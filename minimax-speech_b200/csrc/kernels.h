@@ -5,6 +5,7 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
+#include <vector>
 
 namespace ls {
 
@@ -248,6 +249,36 @@ cudaError_t launch_fsq_encode(const float* x, const float* w, const float* bias,
 // or 0 (and an all-zero mel) when audio_len[b] < 201 or > S.  B <= 65535.
 cudaError_t launch_s3_log_mel(const float* audio, const int* audio_len, const float* filters, int n_mels, float* mel,
                               int* mel_len, int B, long long S, cudaStream_t s);
+// ---- sample-rate conversion and latent stretch (resample.cu) ----
+// The taps of torchaudio.functional.resample (sinc_interp_hann, width 6, rolloff 0.99) with |t| < 6, one row per phase:
+// output sample j = q*N + p is sum_k taps[p][k] * x[q*O + first[p] + k] for k < count[p].  taps: [N][max_taps], fp32.
+struct ResampleTable {
+  int O = 0, N = 0, width = 0, max_taps = 0;  // reduced ratio O / N (orig / new), torchaudio's window half-width
+  std::vector<int> first, count;
+  std::vector<float> taps;
+};
+constexpr long long kResampleMaxTableBytes = 96 << 10;
+constexpr size_t kResampleMaxSmem = 200 << 10;
+inline long long resample_table_bytes(const ResampleTable& t) { return 4LL * t.N * t.max_taps; }
+// LS_OK, LS_ERR_INVALID (a rate <= 0) or LS_ERR_UNSUPPORTED (table over kResampleMaxTableBytes; O, N, width are set).
+// fill = false computes the sizes only.  Host only.
+int resample_table(int orig_freq, int new_freq, ResampleTable* t, bool fill = true);
+struct ResamplePlan {
+  const float* taps = nullptr;  // device [N][stride]
+  const int2* fc = nullptr;     // device [N] (first, count)
+  int O = 0, N = 0, stride = 0, min_first = 0, tile = 0, span = 0;
+  size_t smem = 0;
+};
+// The launch geometry for a table (taps / fc are the caller's to set); LS_ERR_UNSUPPORTED if it needs too much shared memory.
+int resample_plan(const ResampleTable& t, ResamplePlan* plan);
+// audio [B][S_in] with audio_len [B] -> out [B][S_out] (zero past out_len[b] = ceil(N len / O); S_out >= ceil(N S_in / O)).
+// A length < 1 or > S_in gives out_len 0 and a zero row.  B <= 65535, S_in and S_out < 2^31.
+cudaError_t launch_resample(const ResamplePlan& p, const float* audio, const int* audio_len, float* out, int* out_len, int B,
+                            long long S_in, long long S_out, cudaStream_t s);
+// z [B][C][L_in] -> out [B][C][L_out]: row b's first len_in[b] frames linearly stretched to len_out[b] frames
+// (align_corners=False), zero past len_out[b]; invalid lengths give a zero row.
+cudaError_t launch_latent_resize_linear(const float* z, const int* len_in, const int* len_out, float* out, int B, int C,
+                                        int L_in, int L_out, cudaStream_t s);
 // timestep conditioning for nt time values: sinusoidal embedding -> MLP -> per-resnet projections
 struct TimeEmbedParams {
   const float* t;        // [nt] device, or nullptr: the values come from t_host (nt <= 64) inside the kernel parameters

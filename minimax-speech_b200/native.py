@@ -19,6 +19,7 @@ EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create
            "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode", "ls_front_encode_sessions",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
            "ls_s3_create", "ls_s3_create_fp32", "ls_s3_destroy", "ls_s3_code_frames", "ls_s3_quantize", "ls_s3_log_mel",
+           "ls_resampler_create", "ls_resampler_destroy", "ls_resample", "ls_resample_taps", "ls_latent_resize_linear",
            "ls_flow_destroy",
            "ls_flow_estimator_forward", "ls_flow_solve", "ls_dac_create", "ls_dac_destroy", "ls_dac_hop_length",
            "ls_dac_decode", "ls_synthesize_host", "ls_fsq_encode", "ls_mask_to_lengths", "ls_graph_create", "ls_graph_buffer",
@@ -123,7 +124,14 @@ def load():
         lib.ls_s3_code_frames.argtypes = [i32]
         lib.ls_s3_quantize.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, vp]
         lib.ls_s3_log_mel.argtypes = [vp, vp, vp, i32, vp, vp, i32, i64, vp]
-        lib.ls_synthesize_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp, i32, f32, f32, vp, i32, i32, vp]
+        pi32 = C.POINTER(i32)
+        lib.ls_resampler_create.argtypes = [i32, i32, i32, C.POINTER(vp)]
+        lib.ls_resampler_destroy.argtypes = [vp]
+        lib.ls_resampler_destroy.restype = None
+        lib.ls_resample.argtypes = [vp, vp, vp, vp, vp, i32, i64, i64, vp]
+        lib.ls_resample_taps.argtypes = [i32, i32, pi32, pi32, pi32, pi32, vp, vp, vp]
+        lib.ls_latent_resize_linear.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.ls_synthesize_host.argtypes =[vp, vp, vp, vp, vp, vp, vp, i64, vp, i32, f32, f32, vp, i32, i32, vp]
         lib.ls_mask_to_lengths.argtypes = [vp, vp, i32, i32, vp]
         lib.ls_fsq_encode.argtypes = [vp, vp, vp, vp, i64, i32, vp]
         lib.ls_graph_create.argtypes = [vp, vp, vp, i64, vp, i32, f32, f32, i32, i32, i32, vp, C.POINTER(vp)]
@@ -427,6 +435,58 @@ def s3_log_mel(audio, audio_len, filters):
     check(load().ls_s3_log_mel(ptr(audio), ptr(audio_len), ptr(filters), n_mels, ptr(mel), ptr(mel_len), B, S,
                                current_stream_ptr(audio.device)), "ls_s3_log_mel")
     return mel, mel_len
+
+
+def resample_taps(orig_freq, new_freq):
+    """The tap table ls_resample uses for orig_freq -> new_freq (host only, no device needed): dict with the reduced
+    ratio ``O`` / ``N``, torchaudio's ``width``, ``max_taps``, and numpy ``first`` [N], ``count`` [N] (int32) and ``taps``
+    [N, max_taps] (float32, zero-padded).  Raises for a table over 96 KiB (``ls_resample_taps``)."""
+    lib = load()
+    O, N, W, M = (C.c_int32() for _ in range(4))
+    check(lib.ls_resample_taps(int(orig_freq), int(new_freq), C.byref(O), C.byref(N), C.byref(W), C.byref(M), None, None, None),
+          "ls_resample_taps")
+    first, count = np.zeros(N.value, np.int32), np.zeros(N.value, np.int32)
+    taps = np.zeros((N.value, M.value), np.float32)
+    check(lib.ls_resample_taps(int(orig_freq), int(new_freq), None, None, None, None, C.c_void_p(first.ctypes.data),
+                               C.c_void_p(count.ctypes.data), C.c_void_p(taps.ctypes.data)), "ls_resample_taps")
+    return dict(O=O.value, N=N.value, width=W.value, max_taps=M.value, first=first, count=count, taps=taps)
+
+
+class ResamplerHandle:
+    """Owns an ls_resampler*: the tap table of one (orig_freq, new_freq) pair on one device."""
+
+    def __init__(self, orig_freq, new_freq, device):
+        lib = load()
+        self.device = torch.device(device)
+        self.orig_freq, self.new_freq = int(orig_freq), int(new_freq)
+        h = C.c_void_p()
+        with torch.cuda.device(self.device):
+            check(lib.ls_resampler_create(self.orig_freq, self.new_freq, self.device.index or 0, C.byref(h)),
+                  "ls_resampler_create")
+        self._h = h
+
+    def __del__(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h and _lib is not None:
+            _lib.ls_resampler_destroy(h)
+
+    def resample(self, audio, audio_len, S_out):
+        """audio [B, S_in] float32, audio_len [B] int32 (device, contiguous) -> out [B, S_out], out_len [B] int32."""
+        B, S_in = audio.shape
+        out = torch.empty(B, S_out, device=audio.device, dtype=torch.float32)
+        out_len = torch.empty(B, device=audio.device, dtype=torch.int32)
+        check(load().ls_resample(self._h, ptr(audio), ptr(audio_len), ptr(out), ptr(out_len), B, S_in, int(S_out),
+                                 current_stream_ptr(audio.device)), "ls_resample")
+        return out, out_len
+
+
+def latent_resize_linear(z, len_in, len_out, L_out):
+    """z [B, C, L_in] float32, len_in / len_out [B] int32 (device) -> [B, C, L_out] (ls_latent_resize_linear)."""
+    B, Cz, L_in = z.shape
+    out = torch.empty(B, Cz, L_out, device=z.device, dtype=torch.float32)
+    check(load().ls_latent_resize_linear(ptr(z), ptr(len_in), ptr(len_out), ptr(out), B, Cz, L_in, int(L_out),
+                                         current_stream_ptr(z.device)), "ls_latent_resize_linear")
+    return out
 
 
 def mask_to_lengths(mask):

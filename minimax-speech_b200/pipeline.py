@@ -217,12 +217,25 @@ def plan_micro_batches(n_samples, max_batch_samples=None):
     return batches
 
 
+def _load_at(load_audio, path, sample_rate, rate, device):
+    """load_audio(path) as a 1-D float32 tensor at ``rate``: converted on the GPU (``audio.resample``) when ``sample_rate``
+    names another rate, returned on the host either way."""
+    a = torch.as_tensor(load_audio(path), dtype=torch.float32).reshape(-1)
+    if sample_rate is None or int(sample_rate) == rate:
+        return a
+    from . import audio as _audio
+    return _audio.resample(a.to(device), sample_rate, rate).cpu()
+
+
 def extract_latents(paths, load_audio, encoder, device, rank=0, world_size=1, save=True, generator=None,
-                    max_batch_samples=None):
+                    max_batch_samples=None, sample_rate=None):
     """Encode this rank's share of ``paths`` and write ``<stem>_latent2x.pt`` next to each input.
     ``load_audio(path) -> 1-D float tensor`` at ``encoder.sample_rate`` (the reference uses librosa, which is not a
-    dependency here).  Audio is clamped to [-1, 1] (:31) and right-padded to a multiple of the hop (DACVAE.preprocess,
-    model.py:455-462; the reference tool feeds the unpadded signal, so its last latent frame can differ).
+    dependency here), or at ``sample_rate`` when given: the audio is then converted to ``encoder.sample_rate`` on the GPU
+    (``audio.resample``, torchaudio's resampler; the reference tool resamples with librosa, whose result this does not
+    reproduce) and the records describe the converted signal.  Audio is clamped to [-1, 1] (:31) and right-padded to a
+    multiple of the hop (DACVAE.preprocess, model.py:455-462; the reference tool feeds the unpadded signal, so its last
+    latent frame can differ).
 
     By default each file is encoded on its own (like the reference).  ``max_batch_samples`` encodes length-sorted
     micro-batches of at most that many padded samples (batch size x longest file, see ``plan_micro_batches``) with
@@ -234,7 +247,7 @@ def extract_latents(paths, load_audio, encoder, device, rank=0, world_size=1, sa
     mine = paths[start:end]
     padded, n_orig, noise = [], [], []
     for path in mine:
-        audio = torch.clamp(torch.as_tensor(load_audio(path), dtype=torch.float32).reshape(1, 1, -1), -1.0, 1.0)
+        audio = torch.clamp(_load_at(load_audio, path, sample_rate, encoder.sample_rate, device).reshape(1, 1, -1), -1.0, 1.0)
         n_orig.append(audio.shape[-1])
         padded.append(encoder.preprocess(audio))
         L = padded[-1].shape[-1] // encoder.hop_length
@@ -281,10 +294,12 @@ def token_record(tokens, n_samples, path, sample_rate=16000):
             "original_samples": n_samples, "original_path": path}
 
 
-def extract_tokens(paths, load_audio, tokenizer, device, rank=0, world_size=1, save=True, max_batch_samples=None):
+def extract_tokens(paths, load_audio, tokenizer, device, rank=0, world_size=1, save=True, max_batch_samples=None,
+                   sample_rate=None):
     """Tokenize this rank's share of ``paths`` (``shard_files``) with an ``S3TokenizerV2`` and write
     ``<stem>_fsq.pt`` (``token_record``) next to each input.  ``load_audio(path) -> 1-D float tensor`` of 16 kHz mono
-    audio (decoding and resampling stay with the caller).
+    audio, or of audio at ``sample_rate`` when given: it is then converted to 16 kHz on the GPU (``audio.resample``) and
+    the records describe the converted signal.  Decoding stays with the caller.
 
     By default each file is one ``quantize_audio`` call.  ``max_batch_samples`` tokenizes length-sorted micro-batches of
     at most that many padded samples (batch size x longest file, see ``plan_micro_batches``) in one call each, with
@@ -293,7 +308,8 @@ def extract_tokens(paths, load_audio, tokenizer, device, rank=0, world_size=1, s
     import os
     start, end = shard_files(len(paths), rank, world_size)
     mine = paths[start:end]
-    audio = [torch.as_tensor(load_audio(path), dtype=torch.float32).reshape(-1) for path in mine]
+    from .tokenizer import SAMPLE_RATE
+    audio = [_load_at(load_audio, path, sample_rate, SAMPLE_RATE, device) for path in mine]
     recs = [None] * len(mine)
     for batch in plan_micro_batches([a.shape[0] for a in audio], max_batch_samples):
         lens = [audio[i].shape[0] for i in batch]
