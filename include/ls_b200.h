@@ -314,9 +314,13 @@ typedef struct ls_conv_gemm_desc {
 /* plan_out: int32[8] = grid, the largest tile count of any CTA, dual issue, resident weights, activation stages,
  * weight stages, TMA stores, halo mode (all 0 when there is nothing to launch) */
 int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* plan_out, void* stream);
-/* qkv bf16 [B][T][3*H*64] -> out bf16 [B][T][H*64] */
+/* qkv [B][T][3*H*64] -> out [B][T][H*64], bf16 (fp16 = 0) or IEEE half (fp16 = 1); softmax scale 0.125.
+ * lengths int32[B] or NULL (= T); chunk > 0: key j visible to query i iff j < (i/chunk + 1)*chunk.
+ * bias (NULL = none): fp32 relative-position term, score(i, j) += bias[(b*H + h)*bias_bh + i*bias_ld + (T-1-i) + j],
+ * with bias_ld >= 2T-1 and bias_bh >= T*bias_ld (the reads then stay inside B*H*bias_bh floats). */
 int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, int32_t B, int32_t T, int32_t H,
-                          int32_t chunk, void* stream);
+                          int32_t chunk, int32_t fp16, const float* bias, int64_t bias_ld, int64_t bias_bh,
+                          void* stream);
 
 /* Fused transformer-block tail (tblock.cu): att bf16 [R][512], u fp32 [R][256] (updated in place when
  * tail_mode == 0), bf16 weights wo [256][512], w1 [1024][256], w2 [256][1024], wqkv [1536][256], vec = 2560 floats

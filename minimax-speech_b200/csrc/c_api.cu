@@ -775,9 +775,16 @@ int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* 
 }
 
 int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, int32_t B, int32_t T, int32_t H,
-                          int32_t chunk, void* stream) {
+                          int32_t chunk, int32_t fp16, const float* bias, int64_t bias_ld, int64_t bias_bh,
+                          void* stream) {
   return ls::guarded([&] {
     ls::require(qkv && out, "ls_test_attention: null argument");
+    ls::require(B >= 1 && B <= 65535 && T >= 1 && H >= 1 && H <= 65535 && chunk >= 0,
+                "ls_test_attention: B, T, H or chunk out of range");
+    ls::require(fp16 == 0 || fp16 == 1, "ls_test_attention: fp16 must be 0 or 1");
+    if (bias)
+      ls::require(bias_ld >= 2LL * T - 1 && bias_bh >= (long long)T * bias_ld,
+                  "ls_test_attention: bias needs bias_ld >= 2T-1 and bias_bh >= T*bias_ld");
     CUtensorMap m;
     ls::require(ls::make_act_map(&m, qkv, 3 * H * 64, T, B, 3 * H * 64, (long long)T * 3 * H * 64, ATTN_KV),
                 "tensor map qkv", LS_ERR_CUDA);
@@ -785,6 +792,8 @@ int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, in
     ap.B = B, ap.T = T, ap.H = H, ap.lengths = lengths, ap.chunk = chunk;
     ap.scale_log2e = 0.125f * 1.4426950408889634f;
     ap.out = reinterpret_cast<__nv_bfloat16*>(out);
+    ap.bias = bias, ap.bias_ld = bias_ld, ap.bias_bh = bias_bh;
+    ap.fp16 = fp16;
     LS_CUDA(ls::launch_attention(m, ap, (cudaStream_t)stream));
   });
 }

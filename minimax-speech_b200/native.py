@@ -146,7 +146,7 @@ def load():
         lib.ls_profile_end.argtypes = [C.POINTER(ProfileEntry), i32]
         lib.ls_test_tblock.argtypes = [vp] * 10 + [i32, i32, i32, i32, vp, vp]
         lib.ls_test_conv_gemm.argtypes = [C.POINTER(ConvGemmDesc), i32, vp, vp]
-        lib.ls_test_attention.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.ls_test_attention.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp, i64, i64, vp]
         for name in EXPORTS:
             fn = getattr(lib, name)
             if fn.restype is C.c_int:
@@ -154,6 +154,8 @@ def load():
         # the kernel test hooks' SM count and plan arguments (just before the stream) are optional for Python callers
         lib.ls_test_conv_gemm = _plan_args_optional(lib.ls_test_conv_gemm, 1)
         lib.ls_test_tblock = _plan_args_optional(lib.ls_test_tblock, 13)
+        # ... and so are the attention hook's fp16 flag and bias arguments (bf16, no bias)
+        lib.ls_test_attention = _attention_args_optional(lib.ls_test_attention)
         _lib = lib
         return lib
 
@@ -163,6 +165,17 @@ def _plan_args_optional(fn, n_fixed):
     def call(*args):
         if len(args) == n_fixed + 1:
             args = args[:-1] + (0, None, args[-1])
+        return fn(*args)
+    call.__name__ = fn.__name__
+    return call
+
+
+def _attention_args_optional(fn):
+    """fn(qkv, out, lengths, B, T, H, chunk, fp16, bias, bias_ld, bias_bh, stream) also callable as
+    fn(qkv, out, lengths, B, T, H, chunk, stream): bf16 operands, no bias"""
+    def call(*args):
+        if len(args) == 8:
+            args = args[:-1] + (0, None, 0, 0, args[-1])
         return fn(*args)
     call.__name__ = fn.__name__
     return call
