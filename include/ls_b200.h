@@ -89,6 +89,12 @@ int32_t ls_flow_solve(ls_flow* h, const float* mu, const float* mask, const floa
 
 /* ---- DAC-VAE decoder ---- */
 int32_t ls_dac_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out);
+/* fp16-operand mode of the DAC-VAE handle: the same tensor-core kernels with fp16 instead of bf16 GEMM operands (the
+ * folded weights, z, and every Snake / LeakyReLU output a convolution consumes); accumulation stays fp32, the decoder's
+ * residual stream fp16, the encoder's fp32, and the waveform and z / m / logs fp32.  Like ls_dac_create it builds the
+ * decoder, the encoder, or both, from whatever the state dict holds, and the handle takes the same calls (including
+ * ls_graph_create).  A folded weight outside fp16's range (|w| > 65504) fails with LS_ERR_UNSUPPORTED naming the layer. */
+int32_t ls_dac_create_fp16(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out);
 int32_t ls_dac_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out);
 void ls_dac_destroy(ls_dac* h);
 int32_t ls_dac_hop_length(const ls_dac* h);
@@ -310,6 +316,7 @@ typedef struct ls_conv_gemm_desc {
   const float* p1_b;
   int32_t n_store;
   int64_t out_ld, out_shift, out_bstride, out_alloc, out_valid_mul;
+  int32_t fp16; /* 0: bf16 operands and 16-bit outputs (dtype 2), 1: fp16; fp16 outputs (dtype 3) are IEEE half either way */
 } ls_conv_gemm_desc;
 /* plan_out: int32[8] = grid, the largest tile count of any CTA, dual issue, resident weights, activation stages,
  * weight stages, TMA stores, halo mode (all 0 when there is nothing to launch) */

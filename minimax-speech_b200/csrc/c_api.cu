@@ -379,17 +379,27 @@ int32_t ls_flow_solve(ls_flow* h, const float* mu, const float* mask, const floa
   });
 }
 
-int32_t ls_dac_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out) {
+namespace {
+// ls_dac_create / ls_dac_create_fp16: the decoder, the encoder, or both, from whatever the state dict holds
+int32_t dac_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out, bool fp16, const char* fn) {
   return ls::guarded([&] {
-    ls::require(weights && out && n_weights > 0, "ls_dac_create: null argument");
+    ls::require(weights && out && n_weights > 0, std::string(fn) + ": null argument");
     ls::Weights w(weights, n_weights);
     auto h = std::make_unique<ls_dac>();
     const bool has_dec = w.has("decoder.model.0.0.weight_v"), has_enc = w.has("encoder.block.0.0.weight_v");
-    ls::require(has_dec || has_enc, "ls_dac_create: neither decoder.* nor encoder.* weights found", LS_ERR_WEIGHTS);
-    if (has_dec) h->eng = std::make_unique<ls::DacEngine>(w, device);
-    if (has_enc) h->enc = std::make_unique<ls::DacEncEngine>(w, device);
+    ls::require(has_dec || has_enc, std::string(fn) + ": neither decoder.* nor encoder.* weights found", LS_ERR_WEIGHTS);
+    if (has_dec) h->eng = std::make_unique<ls::DacEngine>(w, device, fp16);
+    if (has_enc) h->enc = std::make_unique<ls::DacEncEngine>(w, device, fp16);
     *out = h.release();
   });
+}
+}  // namespace
+
+int32_t ls_dac_create(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out) {
+  return dac_create(weights, n_weights, device, out, false, "ls_dac_create");
+}
+int32_t ls_dac_create_fp16(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out) {
+  return dac_create(weights, n_weights, device, out, true, "ls_dac_create_fp16");
 }
 int32_t ls_dac_create_fp32(const ls_tensor* weights, int32_t n_weights, int32_t device, ls_dac** out) {
   return ls::guarded([&] {
@@ -769,7 +779,8 @@ int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* 
     p.p1_a = d->p1_a, p.p1_b = d->p1_b, p.n_store = d->n_store;
     p.out_ld = d->out_ld, p.out_shift = d->out_shift, p.out_bstride = d->out_bstride, p.out_alloc = d->out_alloc;
     p.out_valid_mul = d->out_valid_mul;
-    p.k_true = d->K, p.tag = 0, p.halo_mode = ls::conv_halo_mode();
+    ls::require(d->fp16 == 0 || d->fp16 == 1, "ls_test_conv_gemm: fp16 must be 0 or 1");
+    p.k_true = d->K, p.tag = 0, p.halo_mode = ls::conv_halo_mode(), p.fp16 = d->fp16;
     LS_CUDA(ls::launch_conv_gemm(a0, a1, w, p, sms, (cudaStream_t)stream, plan_out));
   });
 }

@@ -1315,8 +1315,8 @@ cudaError_t LS_FN(launch_conv_gemm)(const CUtensorMap& mapA0, const CUtensorMap&
   LS_CONV_CASE(ACT_LN_MISH, OUT_F32, OUT1_LN, ADD_GEMM, 0)
   LS_CONV_CASE(ACT_NONE, OUT_NONE, OUT1_COPY, OUT_NONE, 0)
   LS_CONV_CASE(ACT_LN_MISH, OUT_NONE, OUT1_COPY, OUT_NONE, 0)
-#if !LS_HALF_FP16  // (the fp16-operand build serves the flow estimator only)
   // DAC decoder: de_conv_pre | input conv, conv7 | transposed conv | conv1 + residual (x kept / last unit) | final conv
+  // (both builds: the fp16-operand build serves the flow estimator and the fp16 DAC decoder / encoder handles)
   LS_CONV_CASE(ACT_LRELU, OUT_NONE, OUT1_COPY, OUT_NONE, 0)
   LS_CONV_CASE(ACT_LRELU, OUT_NONE, OUT1_SNAKE, OUT_NONE, 0)
   LS_CONV_CASE(ACT_NONE, OUT_F32, OUT1_SNAKE, OUT_NONE, 0)
@@ -1326,7 +1326,6 @@ cudaError_t LS_FN(launch_conv_gemm)(const CUtensorMap& mapA0, const CUtensorMap&
   LS_CONV_CASE(ACT_LRELU, OUT_F16, OUT1_SNAKE, OUT_F16, 0)
   LS_CONV_CASE(ACT_LRELU, OUT_NONE, OUT1_SNAKE, OUT_F16, 0)
   LS_CONV_CASE(ACT_LRELU_TANH, OUT_F32, OUT1_NONE, OUT_NONE, 0)
-#endif
 #undef LS_CONV_CASE
   return launch_instance<-1, -1, -1, -1, -1>(grid, smem, stream, mapA0, mapA1, mapW, *mo0, *mo1, pp, tmem_cols, acc_stride);
 }

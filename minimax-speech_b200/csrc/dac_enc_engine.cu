@@ -17,14 +17,15 @@
 namespace ls {
 namespace {
 
-// first convolution (1 -> C0, k = 7, pad 3) + LeakyReLU(0.1): x fp32 [B][S][C0] and snake(x) bf16 for the first unit.
+// first convolution (1 -> C0, k = 7, pad 3) + LeakyReLU(0.1): x fp32 [B][S][C0] and snake(x) for the first unit, in the
+// handle's 16-bit operand format (fp16 = 1: IEEE half, else bf16).
 // lengths (nullable, latent frames): item b is the samples [0, lengths[b] * hop) of its row; later samples are never
 // read (they count as the convolution's zero padding) and rows from there to S are written as zeros.
 __global__ void __launch_bounds__(128) enc_in_conv_kernel(const float* __restrict__ audio, const int* __restrict__ lengths,
                                                           int hop, const float* __restrict__ w,
                                                           const float* __restrict__ bias, const float* __restrict__ alpha,
                                                           const float* __restrict__ ialpha, float* __restrict__ x,
-                                                          __nv_bfloat16* __restrict__ sn, int S, int C0) {
+                                                          __nv_bfloat16* __restrict__ sn, int S, int C0, int fp16) {
   const int t = blockIdx.x * 128 + threadIdx.x;
   const int b = blockIdx.y;
   if (t >= S) return;
@@ -60,7 +61,8 @@ __global__ void __launch_bounds__(128) enc_in_conv_kernel(const float* __restric
     float s4[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) s4[j] = snake_f(vv[j], alpha[n + j], ialpha[n + j]);
-    pk[0] = pack_bf16x2(s4[0], s4[1]), pk[1] = pack_bf16x2(s4[2], s4[3]);
+    if (fp16) pk[0] = pack_f16x2(s4[0], s4[1]), pk[1] = pack_f16x2(s4[2], s4[3]);
+    else pk[0] = pack_bf16x2(s4[0], s4[1]), pk[1] = pack_bf16x2(s4[2], s4[3]);
     *reinterpret_cast<uint2*>(so + n) = make_uint2(pk[0], pk[1]);
   }
 }
@@ -94,8 +96,8 @@ __global__ void enc_post_kernel(const float* __restrict__ y, const int* __restri
   z[o] = noise ? am + noise[o] * expf(al) : am;
 }
 
-// stride-s WNConv1d weight_v [N][C][2s] -> 3-tap polyphase bf16 [3][N][s*C] (see the header comment)
-PackedLinear pack_wn_down(Arena& a, const Weights& w, const std::string& p, int stride) {
+// stride-s WNConv1d weight_v [N][C][2s] -> 3-tap polyphase 16-bit [3][N][s*C] (see the header comment)
+PackedLinear pack_wn_down(Arena& a, const Weights& w, const std::string& p, int stride, bool fp16) {
   const ls_tensor& v = w.get(p + ".weight_v");
   const ls_tensor& g = w.get(p + ".weight_g");
   const ls_tensor& b = w.get(p + ".bias");
@@ -106,7 +108,7 @@ PackedLinear pack_wn_down(Arena& a, const Weights& w, const std::string& p, int 
   pl.N = N, pl.K = stride * C, pl.taps = 3, pl.block_n = pick_block_n(N);
   pl.w_off = a.reserve((size_t)3 * N * pl.K * 2);
   __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(a.host(pl.w_off));
-  for (size_t i = 0; i < (size_t)3 * N * pl.K; ++i) dst[i] = __float2bfloat16(0.f);
+  for (size_t i = 0; i < (size_t)3 * N * pl.K; ++i) dst[i] = __float2bfloat16(0.f);  // 0 has the same bits in fp16
   const size_t per = (size_t)C * k2;
   for (int n = 0; n < N; ++n) {
     double ss = 0;
@@ -117,7 +119,7 @@ PackedLinear pack_wn_down(Arena& a, const Weights& w, const std::string& p, int 
         const int k = q * stride + r + pad;
         if (k < 0 || k >= k2) continue;
         for (int c = 0; c < C; ++c)
-          dst[((size_t)(q + 1) * N + n) * pl.K + (size_t)r * C + c] = __float2bfloat16(v.data[(n * (size_t)C + c) * k2 + k] * scale);
+          dst[((size_t)(q + 1) * N + n) * pl.K + (size_t)r * C + c] = dac_w16(v.data[(n * (size_t)C + c) * k2 + k] * scale, fp16, p);
       }
   }
   pl.bias_off = a.put_f32(b.data, N);
@@ -140,7 +142,7 @@ DacEncEngine::~DacEncEngine() {
   if (ws_base_) cudaFree(ws_base_);
 }
 
-DacEncEngine::DacEncEngine(const Weights& w, int device) : device_(device) {
+DacEncEngine::DacEncEngine(const Weights& w, int device, bool fp16) : device_(device), fp16_(fp16 ? 1 : 0) {
   LS_CUDA(cudaSetDevice(device));
   cudaDeviceProp prop;
   LS_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -183,13 +185,13 @@ DacEncEngine::DacEncEngine(const Weights& w, int device) : device_(device) {
     for (int j = 0; j < 3; ++j) {
       const std::string q = p + "." + std::to_string(j) + ".block";
       snake(q + ".0.alpha", c, &st.unit[j].a0, &st.unit[j].ia0);
-      st.unit[j].conv7 = pack_wn_conv(arena_, w, q + ".1.0");
+      st.unit[j].conv7 = pack_wn_conv(arena_, w, q + ".1.0", fp16);
       snake(q + ".2.alpha", c, &st.unit[j].a2, &st.unit[j].ia2);
-      st.unit[j].conv1 = pack_wn_conv(arena_, w, q + ".3.0");
+      st.unit[j].conv1 = pack_wn_conv(arena_, w, q + ".3.0", fp16);
       require(st.unit[j].conv7.taps == 7 && st.unit[j].conv1.taps == 1, "unexpected ResidualUnit at " + q, LS_ERR_UNSUPPORTED);
     }
     snake(p + ".3.alpha", c, &st.a_dn, &st.ia_dn);
-    st.down = pack_wn_down(arena_, w, p + ".4.0", st.stride);
+    st.down = pack_wn_down(arena_, w, p + ".4.0", st.stride, fp16);
     hop_ *= st.stride;
     c *= 2;
     stages_.push_back(st);
@@ -197,7 +199,7 @@ DacEncEngine::DacEncEngine(const Weights& w, int device) : device_(device) {
   const int n = (int)stages_.size();
   require(n >= 1 && n <= 5, "DAC encoder must have 1..5 downsampling stages", LS_ERR_UNSUPPORTED);
   snake("encoder.block." + std::to_string(n + 1) + ".alpha", c, &final_alpha_, &final_ialpha_);
-  final_ = pack_wn_conv(arena_, w, "encoder.block." + std::to_string(n + 2) + ".0");
+  final_ = pack_wn_conv(arena_, w, "encoder.block." + std::to_string(n + 2) + ".0", fp16);
   latent_ = final_.N;
   require(final_.taps == 3 && latent_ % 16 == 0, "unexpected encoder head", LS_ERR_UNSUPPORTED);
   const ls_tensor& vp = w.get("en_conv_post.0.weight_v");
@@ -291,14 +293,14 @@ void DacEncEngine::encode(const float* audio, const int* lengths, const float* n
     p.bias = w.bias, p.chan_mod = w.N, p.n_store = w.N;
     p.out_ld = w.N, p.out_shift = 0, p.out_bstride = rows * w.N, p.out_alloc = rows * w.N;
     p.out_valid_mul = lengths ? (long long)rate * w.N : w.N;
-    p.k_true = w.K, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0;
+    p.k_true = w.K, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0, p.fp16 = fp16_;
     LS_CUDA(launch_conv_gemm(a, a, w.map, p, num_sms_, s));
   };
 
   count_launch();
   enc_in_conv_kernel<<<dim3((S + 127) / 128, B), 128, 0, s>>>(audio, lengths, hop_, f32(in_w_), f32(in_b_),
                                                             f32(stages_[0].unit[0].a0), f32(stages_[0].unit[0].ia0), x,
-                                                            ws<__nv_bfloat16>(o_sA_), S, dim0_);
+                                                            ws<__nv_bfloat16>(o_sA_), S, dim0_, fp16_);
   LS_CUDA(cudaGetLastError());
   long long rows = S;
   int rate = hop_;

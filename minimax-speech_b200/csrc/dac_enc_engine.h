@@ -11,7 +11,9 @@ namespace ls {
 // tensor-core path: every ResidualUnit convolution and every downsampling convolution is a conv_gemm launch.
 class DacEncEngine {
  public:
-  DacEncEngine(const Weights& w, int device);
+  // fp16: fp16 instead of bf16 GEMM operands (weights and the Snake outputs the convolutions consume); accumulation,
+  // the residual stream and z / m / logs stay fp32
+  DacEncEngine(const Weights& w, int device, bool fp16 = false);
   ~DacEncEngine();
   // audio [B,1,S] fp32 (S a multiple of the hop) -> z, m, logs [B,latent,S/hop] fp32; noise nullable ([B,latent,S/hop]).
   // lengths (device int32 [B], nullable): latent frames per clip; clip b is encoded as if alone at lengths[b] * hop
@@ -39,7 +41,7 @@ class DacEncEngine {
   template <typename T>
   T* ws(size_t off) const { return reinterpret_cast<T*>(ws_base_ + off); }
 
-  int device_ = 0, num_sms_ = 148, latent_ = 80, hop_ = 1, dim0_ = 64;
+  int device_ = 0, num_sms_ = 148, latent_ = 80, hop_ = 1, dim0_ = 64, fp16_ = 0;
   Arena arena_;
   size_t in_w_ = 0, in_b_ = 0;       // first conv (1 -> dim0, k = 7), fp32 [dim0][7] + bias
   size_t post_w_ = 0, post_b_ = 0;   // en_conv_post folded, fp32 [2*latent][latent] + bias

@@ -4,15 +4,16 @@
 // (DecoderBlock), :107-143 (ResidualUnit), with every generator Conv1d followed by LeakyReLU(0.1)
 // (the shadowing WNConv1d at model.py:509-514).  weight_norm (layers.py:9-14) is folded once here.
 // All convolutions run as conv_gemm launches; Snake1d (layers.py:18-33) is never a pass of its own: each
-// epilogue emits snake(x) for the *next* convolution as its bf16 secondary output.
+// epilogue emits snake(x) for the *next* convolution as its 16-bit secondary output (bf16, or fp16 for a handle
+// built with fp16 operands).
 #include <cmath>
 
 #include "dac_engine.h"
 
 namespace ls {
 
-// Conv1d weight_v [N][K][taps] with weight_g [N] -> folded bf16 [taps][Npad][K]
-PackedLinear pack_wn_conv(Arena& a, const Weights& w, const std::string& p, int n_pad_to) {
+// Conv1d weight_v [N][K][taps] with weight_g [N] -> folded 16-bit [taps][Npad][K]
+PackedLinear pack_wn_conv(Arena& a, const Weights& w, const std::string& p, bool fp16, int n_pad_to) {
   const ls_tensor& v = w.get(p + ".weight_v");
   const ls_tensor& g = w.get(p + ".weight_g");
   const ls_tensor& b = w.get(p + ".bias");
@@ -25,7 +26,7 @@ PackedLinear pack_wn_conv(Arena& a, const Weights& w, const std::string& p, int 
   pl.block_n = pick_block_n(pl.N);
   pl.w_off = a.reserve((size_t)pl.taps * pl.N * pl.K * 2);
   __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(a.host(pl.w_off));
-  for (size_t i = 0; i < (size_t)pl.taps * pl.N * pl.K; ++i) dst[i] = __float2bfloat16(0.f);
+  for (size_t i = 0; i < (size_t)pl.taps * pl.N * pl.K; ++i) dst[i] = __float2bfloat16(0.f);  // 0 has the same bits in fp16
   const size_t per = (size_t)pl.K * pl.taps;
   for (int n = 0; n < N; ++n) {
     double ss = 0;
@@ -33,7 +34,7 @@ PackedLinear pack_wn_conv(Arena& a, const Weights& w, const std::string& p, int 
     const float scale = g.data[n] / (float)std::sqrt(ss);
     for (int k = 0; k < pl.K; ++k)
       for (int t = 0; t < pl.taps; ++t)
-        dst[((size_t)t * pl.N + n) * pl.K + k] = __float2bfloat16(v.data[(n * (size_t)pl.K + k) * pl.taps + t] * scale);
+        dst[((size_t)t * pl.N + n) * pl.K + k] = dac_w16(v.data[(n * (size_t)pl.K + k) * pl.taps + t] * scale, fp16, p);
   }
   std::vector<float> bias(pl.N, 0.f);
   for (int n = 0; n < N; ++n) bias[n] = b.data[n];
@@ -50,10 +51,10 @@ void finalize_linear(const Arena& a, PackedLinear& pl) {
 
 namespace {
 
-// ConvTranspose1d weight_v [Cin][Cout][2s], weight_g [Cin] -> two-tap polyphase GEMM, bf16 [2][s*Cout][Cin]:
+// ConvTranspose1d weight_v [Cin][Cout][2s], weight_g [Cin] -> two-tap polyphase GEMM, 16-bit [2][s*Cout][Cin]:
 //   out[q*s + phi - pad] = in[q] . W[:, :, phi] + in[q-1] . W[:, :, phi + s]        (model.py:255-262)
 // tap 0 multiplies in[q-1], tap 1 multiplies in[q]  (A row = q + tap - 1).
-PackedLinear pack_wn_convT(Arena& a, const Weights& w, const std::string& p, int stride) {
+PackedLinear pack_wn_convT(Arena& a, const Weights& w, const std::string& p, int stride, bool fp16) {
   const ls_tensor& v = w.get(p + ".weight_v");
   const ls_tensor& g = w.get(p + ".weight_g");
   const ls_tensor& b = w.get(p + ".bias");
@@ -73,8 +74,8 @@ PackedLinear pack_wn_convT(Arena& a, const Weights& w, const std::string& p, int
       for (int phi = 0; phi < stride; ++phi) {
         const float w_q = v.data[(c * (size_t)cout + n) * k2 + phi] * scale;            // multiplies in[q]
         const float w_qm1 = v.data[(c * (size_t)cout + n) * k2 + phi + stride] * scale;  // multiplies in[q-1]
-        dst[((size_t)0 * pl.N + phi * cout + n) * cin + c] = __float2bfloat16(w_qm1);
-        dst[((size_t)1 * pl.N + phi * cout + n) * cin + c] = __float2bfloat16(w_q);
+        dst[((size_t)0 * pl.N + phi * cout + n) * cin + c] = dac_w16(w_qm1, fp16, p);
+        dst[((size_t)1 * pl.N + phi * cout + n) * cin + c] = dac_w16(w_q, fp16, p);
       }
   }
   pl.bias_off = a.put_f32(b.data, cout);
@@ -108,7 +109,7 @@ DacEngine::~DacEngine() {
   if (ws_base_) cudaFree(ws_base_);
 }
 
-DacEngine::DacEngine(const Weights& w, int device) : device_(device) {
+DacEngine::DacEngine(const Weights& w, int device, bool fp16) : device_(device), fp16_(fp16 ? 1 : 0) {
   LS_CUDA(cudaSetDevice(device));
   cudaDeviceProp prop;
   LS_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -123,8 +124,8 @@ DacEngine::DacEngine(const Weights& w, int device) : device_(device) {
     *ia_off = arena_.put_f32(ia.data(), c);
   };
 
-  pre_ = pack_wn_conv(arena_, w, "de_conv_pre.0");
-  in_ = pack_wn_conv(arena_, w, "decoder.model.0.0");
+  pre_ = pack_wn_conv(arena_, w, "de_conv_pre.0", fp16);
+  in_ = pack_wn_conv(arena_, w, "decoder.model.0.0", fp16);
   latent_ = pre_.K;
   dim_ = in_.N;
   require(pre_.taps == 1 && in_.taps == 7 && latent_ % 16 == 0 && dim_ % 16 == 0, "unexpected DAC decoder stem",
@@ -138,13 +139,13 @@ DacEngine::DacEngine(const Weights& w, int device) : device_(device) {
     st.cin = c, st.cout = c / 2;
     require(st.cout % 16 == 0, "decoder channel count must stay a multiple of 16", LS_ERR_UNSUPPORTED);
     snake(p + ".0.alpha", c, &st.a_in, &st.ia_in);
-    st.up = pack_wn_convT(arena_, w, p + ".1", st.stride);
+    st.up = pack_wn_convT(arena_, w, p + ".1", st.stride, fp16);
     for (int j = 0; j < 3; ++j) {
       const std::string q = p + "." + std::to_string(j + 2) + ".block";
       snake(q + ".0.alpha", st.cout, &st.unit[j].a0, &st.unit[j].ia0);
-      st.unit[j].conv7 = pack_wn_conv(arena_, w, q + ".1.0");
+      st.unit[j].conv7 = pack_wn_conv(arena_, w, q + ".1.0", fp16);
       snake(q + ".2.alpha", st.cout, &st.unit[j].a2, &st.unit[j].ia2);
-      st.unit[j].conv1 = pack_wn_conv(arena_, w, q + ".3.0");
+      st.unit[j].conv1 = pack_wn_conv(arena_, w, q + ".3.0", fp16);
       require(st.unit[j].conv7.taps == 7 && st.unit[j].conv1.taps == 1, "unexpected ResidualUnit at " + q,
               LS_ERR_UNSUPPORTED);
     }
@@ -156,7 +157,7 @@ DacEngine::DacEngine(const Weights& w, int device) : device_(device) {
   const int n = (int)stages_.size();
   require(n >= 1 && n <= 5, "DAC decoder must have 1..5 upsampling stages", LS_ERR_UNSUPPORTED);
   snake("decoder.model." + std::to_string(n + 1) + ".alpha", c, &final_alpha_, &final_ialpha_);
-  final_ = pack_wn_conv(arena_, w, "decoder.model." + std::to_string(n + 2) + ".0", 16);
+  final_ = pack_wn_conv(arena_, w, "decoder.model." + std::to_string(n + 2) + ".0", fp16, 16);
   out_ch_ = (int)w.get("decoder.model." + std::to_string(n + 2) + ".0.bias").shape[0];
   require(out_ch_ == 1 && final_.taps == 7, "only mono output (d_out=1) is covered", LS_ERR_UNSUPPORTED);
 
@@ -252,11 +253,11 @@ void DacEngine::decode(const float* z, const int* lengths, float* wav, int B, in
       p.out_ld = w.N, p.out_shift = 0, p.out_bstride = rows * w.N, p.out_alloc = rows * w.N;
       p.out_valid_mul = (long long)rate * w.N;
     }
-    p.k_true = w.K, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0;
+    p.k_true = w.K, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0, p.fp16 = fp16_;
     LS_CUDA(launch_conv_gemm(a, a, w.map, p, num_sms_, s));
   };
 
-  LS_CUDA(launch_pack_nct(z, ws<__nv_bfloat16>(o_zt_), B, latent_, L, (long long)latent_ * L, latent_, 0, lengths, s));
+  LS_CUDA(launch_pack_nct(z, ws<__nv_bfloat16>(o_zt_), B, latent_, L, (long long)latent_ * L, latent_, 0, lengths, s, fp16_));
   {  // de_conv_pre: 1x1 + LeakyReLU
     ConvGemmParams p{};
     p.act = ACT_LRELU, p.out1 = ws<void>(o_a0_), p.out1_mode = OUT1_COPY;
@@ -271,8 +272,8 @@ void DacEngine::decode(const float* z, const int* lengths, float* wav, int B, in
   long long rows = L;
   int rate = 1;
   // residual stream x of the five stages: written by the transposed conv, read + rewritten by each unit's conv1.
-  // Kept as fp16 (11 significand bits; the operands the convolutions consume are bf16 anyway): the thin stages are
-  // bound by the bytes their epilogues move, and x was half of them as fp32.  -DLS_DAC_X_F32=1 keeps it fp32.
+  // Kept as fp16 (11 significand bits, no fewer than the 16-bit operands the convolutions consume): the thin stages
+  // are bound by the bytes their epilogues move, and x was half of them as fp32.  -DLS_DAC_X_F32=1 keeps it fp32.
 #ifndef LS_DAC_X_F32
 #define LS_DAC_X_F32 0
 #endif
@@ -298,7 +299,7 @@ void DacEngine::decode(const float* z, const int* lengths, float* wav, int B, in
       p.n_store = st.up.N;
       p.out_ld = st.up.N, p.out_shift = -(long long)padT * st.cout;
       p.out_bstride = rows * st.cout, p.out_alloc = rows * st.cout, p.out_valid_mul = (long long)rate * st.cout;
-      p.k_true = st.cin, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0;
+      p.k_true = st.cin, p.tag = 1, p.halo_mode = halo ? conv_halo_mode() : 0, p.fp16 = fp16_;
       LS_CUDA(launch_conv_gemm(pl.sA[i].up, pl.sA[i].up, st.up.map, p, num_sms_, s));
     }
     static const int dils[3] = {1, 3, 9};

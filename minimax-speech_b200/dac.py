@@ -17,7 +17,7 @@ class DACVAEDecoder(nn.Module):
     def __init__(self, latent_dim=80, decoder_dim=1536, decoder_rates=(5, 4, 4, 3, 2), sample_rate=24000,
                  d_out=1, weight_seed=0, precision="bf16", **_ignored):
         super().__init__()
-        self.precision = native.check_precision(precision)
+        self.precision = native.check_precision(precision, fp16_ok=True)
         if d_out != 1:
             raise NotImplementedError("mono output only (configx2.yml: d_out=1)")
         self.latent_dim, self.decoder_dim, self.decoder_rates = latent_dim, decoder_dim, list(decoder_rates)
@@ -72,12 +72,13 @@ class DACVAEDecoder(nn.Module):
 class DACVAEEncoder(nn.Module):
     """``DACVAE.encode`` (dac-vae/model.py:469-483) -- SURVEY section 8 row f-3, the path the reference's multi-GPU
     latent extraction tool runs (extract_dac_latents.py:20-54).  precision="bf16": tensor-core path (every
-    ResidualUnit and downsampling convolution is an implicit-GEMM launch); "fp32": validation mode."""
+    ResidualUnit and downsampling convolution is an implicit-GEMM launch); "fp16": the same path with fp16 GEMM
+    operands; "fp32": validation mode."""
 
     def __init__(self, encoder_dim=64, encoder_rates=(2, 3, 4, 4, 5), latent_dim=80, sample_rate=24000, d_in=1,
                  weight_seed=0, precision="bf16", **_ignored):
         super().__init__()
-        native.check_precision(precision)
+        native.check_precision(precision, fp16_ok=True)
         if d_in != 1:
             raise NotImplementedError("mono input only (configx2.yml: d_in=1)")
         self.precision, self.latent_dim, self.sample_rate = precision, latent_dim, sample_rate
@@ -97,7 +98,7 @@ class DACVAEEncoder(nn.Module):
         device = torch.device(device)
         if device.type != "cuda":
             raise RuntimeError("the B200 hot path runs on CUDA tensors only (no CPU fallback)")
-        if self._handle is None or self._handle.device != device:
+        if self._handle is None or self._handle.device != device or self._handle.precision != self.precision:
             self._handle = native.DacHandle(self.state_dict(), device, self.precision)
         return self._handle
 

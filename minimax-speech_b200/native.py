@@ -14,7 +14,7 @@ ACT_NONE, ACT_LRELU, ACT_GELU, ACT_LN_MISH, ACT_LRELU_TANH = range(5)
 OUT_NONE, OUT_F32, OUT_BF16 = range(3)
 OUT1_NONE, OUT1_LN, OUT1_COPY, OUT1_SNAKE = range(4)
 
-EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create", "ls_flow_create_fp16", "ls_flow_create_fp32", "ls_dac_create_fp32", "ls_dac_encode",
+EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create", "ls_flow_create_fp16", "ls_flow_create_fp32", "ls_dac_create_fp32", "ls_dac_create_fp16", "ls_dac_encode",
            "ls_dac_encode_lengths",
            "ls_front_create", "ls_front_create_fp32", "ls_front_destroy", "ls_front_encode", "ls_front_encode_sessions",
            "ls_speaker_create", "ls_speaker_create_fp32", "ls_speaker_destroy", "ls_speaker_encode",
@@ -50,6 +50,7 @@ class ConvGemmDesc(C.Structure):
         ("n_store", C.c_int32),
         ("out_ld", C.c_int64), ("out_shift", C.c_int64), ("out_bstride", C.c_int64), ("out_alloc", C.c_int64),
         ("out_valid_mul", C.c_int64),
+        ("fp16", C.c_int32),  # 0 (the default of a fresh descriptor): bf16 operands; 1: fp16
     ]
 
 
@@ -95,6 +96,7 @@ def load():
         lib.ls_flow_create_fp32.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_flow_create_fp16.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_dac_create_fp32.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
+        lib.ls_dac_create_fp16.argtypes = [C.POINTER(LsTensor), i32, i32, C.POINTER(vp)]
         lib.ls_flow_destroy.argtypes = [vp]
         lib.ls_flow_destroy.restype = None
         lib.ls_flow_estimator_forward.argtypes = [vp] * 8 + [i32, i32, i32, vp]
@@ -229,13 +231,15 @@ def tensor_table(state_dict):
 
 def check_precision(precision, fp16_ok=False):
     """"bf16": tensor-core path (bf16 operands, fp32 accumulation; latents within about 1e-2 of the fp32 reference);
-    "fp16" (flow estimator only): the same tensor-core path with fp16 operands -- the reference's own half-precision
-    format -- at the same speed, about 2e-3 from the fp32 reference;
+    "fp16" (the flow estimator and the DAC-VAE decoder / encoder, callers pass fp16_ok=True): the same tensor-core path
+    with fp16 operands -- the reference's own half-precision format -- with 3 more mantissa bits, at the speed of bf16
+    for the flow estimator and 1-5 % slower for the DAC (DESIGN section 2);
     "fp32": validation mode, fp32 end to end on the CUDA cores (within 1e-4)."""
     if precision not in ("bf16", "fp16", "fp32"):
         raise ValueError(f"precision must be 'bf16', 'fp16' or 'fp32', not {precision!r}")
     if precision == "fp16" and not fp16_ok:
-        raise ValueError("precision='fp16' (fp16 GEMM operands) is available for the flow estimator only")
+        raise ValueError("precision='fp16' (fp16 GEMM operands) is available for the flow estimator "
+                         "(CausalConditionalDecoder) and the DAC-VAE decoder / encoder (DACVAEDecoder, DACVAEEncoder) only")
     return precision
 
 
@@ -401,12 +405,13 @@ class DacHandle:
     def __init__(self, state_dict, device, precision="bf16"):
         lib = load()
         self.device = torch.device(device)
-        self.precision = check_precision(precision)
+        self.precision = check_precision(precision, fp16_ok=True)
         arr, keep = tensor_table(state_dict)
         h = C.c_void_p()
-        create = lib.ls_dac_create if precision == "bf16" else lib.ls_dac_create_fp32
+        create, name = {"bf16": (lib.ls_dac_create, "ls_dac_create"), "fp16": (lib.ls_dac_create_fp16, "ls_dac_create_fp16"),
+                        "fp32": (lib.ls_dac_create_fp32, "ls_dac_create_fp32")}[precision]
         with torch.cuda.device(self.device):
-            check(create(arr, len(state_dict), self.device.index or 0, C.byref(h)), "ls_dac_create")
+            check(create(arr, len(state_dict), self.device.index or 0, C.byref(h)), name)
         self._h = h
         from . import ops
         self.key = ops.register_handle(self)

@@ -49,7 +49,7 @@ class Synthesizer:
         key = (str(dev), B, T, int(n_timesteps), float(temperature), bool(streaming))
         g = self._graphs.get(key)
         if g is None:
-            if self.cfm.estimator.precision == "fp32" or self.dac.precision != "bf16":
+            if self.cfm.estimator.precision == "fp32" or self.dac.precision == "fp32":
                 raise NotImplementedError("CUDA-graph replay covers the tensor-core path (precision 'bf16' / 'fp16')")
             g = native.GraphHandle(self.cfm.estimator.handle(dev), self.dac.handle(dev), self.cfm._noise_on(dev)[0],
                                    self.cfm._t_span(n_timesteps).numpy(), temperature, self.cfm.inference_cfg_rate,
