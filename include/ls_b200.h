@@ -287,7 +287,8 @@ int32_t ls_profile_end(ls_profile_entry* out, int32_t n_entries);
  * while it is set (NULL clears it).  Not used by any product path. */
 int32_t ls_debug_set_buffer(void* dev_ptr, int64_t bytes);
 
-/* ---- kernel-level hooks used by the kernel tests (tests/test_kernels_gpu.py, tests/test_kernel_plans_gpu.py) ----
+/* ---- kernel-level hooks used by the kernel tests (tests/test_kernels_gpu.py, tests/test_kernel_plans_gpu.py,
+ * tests/test_estimator_kernels_gpu.py) ----
  * Test-only: not part of the product surface, no engine calls them.  num_sms: the SM count the launch plans for
  * (0 = the device's own; a value outside [0, device SMs] is refused with LS_ERR_INVALID), so that small shapes reach
  * the plans a full-size launch takes.  plan_out (may be NULL) receives the plan the launch used. */
@@ -317,6 +318,16 @@ typedef struct ls_conv_gemm_desc {
   int32_t n_store;
   int64_t out_ld, out_shift, out_bstride, out_alloc, out_valid_mul;
   int32_t fp16; /* 0: bf16 operands and 16-bit outputs (dtype 2), 1: fp16; fp16 outputs (dtype 3) are IEEE half either way */
+  int32_t zero_skipped; /* 1: tiles that are all padding still store zeros at their output positions */
+  /* Fused residual GEMM (res_w != NULL, no addend): the epilogue adds R = [res_a0 | res_a1] . res_w^T + res_bias, a
+   * 1x1 convolution computed in the same launch.  res_a0 bf16 [B][T_in][res_a0_C], optional res_a1 [B][T_in][res_a1_C]
+   * (res_a0_C % 64 == 0 then), res_w [N][res_K] with res_K = res_a0_C + res_a1_C, res_bias fp32 [N]. */
+  const void* res_a0;
+  const void* res_a1;
+  int32_t res_a0_C, res_a1_C;
+  const void* res_w;
+  int32_t res_K;
+  const float* res_bias;
 } ls_conv_gemm_desc;
 /* plan_out: int32[8] = grid, the largest tile count of any CTA, dual issue, resident weights, activation stages,
  * weight stages, TMA stores, halo mode (all 0 when there is nothing to launch) */
@@ -332,10 +343,20 @@ int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, in
 /* Fused transformer-block tail (tblock.cu): att bf16 [R][512], u fp32 [R][256] (updated in place when
  * tail_mode == 0), bf16 weights wo [256][512], w1 [1024][256], w2 [256][1024], wqkv [1536][256], vec = 2560 floats
  * (bo, g3, be3, b1, b2, g1n, be1n).  tail_mode 0 -> qkv_out bf16 [R][1536]; 1 -> tail_out bf16 [R][256].
- * plan_out: int32[2] = grid, the largest tile count of any CTA. */
+ * fp16 = 1: every 16-bit operand and output is IEEE half instead of bf16.  no_skip = 1: tiles that hold only padding
+ * rows are processed too.  plan_out: int32[2] = grid, the largest tile count of any CTA. */
 int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1, const void* w2, const void* wqkv,
                        const float* vec, void* qkv_out, void* tail_out, const int32_t* lengths, int32_t R, int32_t T,
-                       int32_t tail_mode, int32_t num_sms, int32_t* plan_out, void* stream);
+                       int32_t tail_mode, int32_t fp16, int32_t no_skip, int32_t num_sms, int32_t* plan_out,
+                       void* stream);
+/* GroupNorm(G) + Mish (elementwise.cu) on fp32 x [B][T][C]: statistics per (batch row, group) over the row's valid frames
+ * (lengths int32[B], clamped to T, or NULL = T) into stats (B*G float pairs of scratch), then on valid frames
+ * y = mish(GroupNorm(x) * gamma + beta) + temb[b*temb_bstride + c] (temb may be NULL) + addend (fp32 [B][T][C], may be
+ * NULL), and 0 on padding frames.  y goes to out_f32 and / or out_h (bf16, or IEEE half when fp16 = 1); either may be
+ * NULL.  C must be a multiple of 4G and C/G of 32. */
+int32_t ls_test_groupnorm_mish(const float* x, void* stats, const float* gamma, const float* beta, const float* temb,
+                               int64_t temb_bstride, const float* addend, float* out_f32, void* out_h, int32_t B,
+                               int32_t C, int32_t T, int32_t G, const int32_t* lengths, int32_t fp16, void* stream);
 
 #ifdef __cplusplus
 }

@@ -781,6 +781,26 @@ int32_t ls_test_conv_gemm(const ls_conv_gemm_desc* d, int32_t num_sms, int32_t* 
     p.out_valid_mul = d->out_valid_mul;
     ls::require(d->fp16 == 0 || d->fp16 == 1, "ls_test_conv_gemm: fp16 must be 0 or 1");
     p.k_true = d->K, p.tag = 0, p.halo_mode = ls::conv_halo_mode(), p.fp16 = d->fp16;
+    p.zero_skipped = d->zero_skipped;
+    if (d->res_w) {  // the fused residual GEMM, set up as flow_engine.cu does (128-row activation boxes whatever the halo mode)
+      ls::require(d->res_a0 != nullptr && !d->addend && d->res_K == d->res_a0_C + d->res_a1_C &&
+                      (d->res_a1 == nullptr || d->res_a0_C % 64 == 0),
+                  "ls_test_conv_gemm: the residual GEMM needs res_a0, no addend, res_K = res_a0_C + res_a1_C and "
+                  "res_a0_C % 64 == 0 with two sources");
+      ls::require(ls::make_act_map(&p.res_a0, d->res_a0, d->res_a0_C, d->T_in, d->B, d->res_a0_C,
+                                   (long long)d->T_in * d->res_a0_C, 128),
+                  "tensor map res_a0", LS_ERR_CUDA);
+      if (d->res_a1)
+        ls::require(ls::make_act_map(&p.res_a1, d->res_a1, d->res_a1_C, d->T_in, d->B, d->res_a1_C,
+                                     (long long)d->T_in * d->res_a1_C, 128),
+                    "tensor map res_a1", LS_ERR_CUDA);
+      else
+        p.res_a1 = p.res_a0;
+      ls::require(ls::make_weight_map(&p.res_w, d->res_w, d->res_K, d->N, d->block_n), "tensor map res_w", LS_ERR_CUDA);
+      p.addend = nullptr, p.addend_dtype = ls::ADD_GEMM;
+      p.res_kb = (d->res_K + 63) / 64, p.res_split = d->res_a1 ? d->res_a0_C / 64 : p.res_kb, p.res_k_true = d->res_K;
+      p.res_bias = d->res_bias;
+    }
     LS_CUDA(ls::launch_conv_gemm(a0, a1, w, p, sms, (cudaStream_t)stream, plan_out));
   });
 }
@@ -811,9 +831,11 @@ int32_t ls_test_attention(const void* qkv, void* out, const int32_t* lengths, in
 
 int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1, const void* w2, const void* wqkv,
                        const float* vec, void* qkv_out, void* tail_out, const int32_t* lengths, int32_t R, int32_t T,
-                       int32_t tail_mode, int32_t num_sms, int32_t* plan_out, void* stream) {
+                       int32_t tail_mode, int32_t fp16, int32_t no_skip, int32_t num_sms, int32_t* plan_out,
+                       void* stream) {
   return ls::guarded([&] {
     ls::require(att && u && wo && w1 && w2 && wqkv && vec, "ls_test_tblock: null argument");
+    ls::require(fp16 == 0 || fp16 == 1, "ls_test_tblock: fp16 must be 0 or 1");
     const int sms = test_hook_sms(num_sms, "ls_test_tblock");
     ls::require(tail_mode != 1 ? qkv_out != nullptr : tail_out != nullptr, "ls_test_tblock: missing output");
     ls::TBlockMaps m;
@@ -832,8 +854,19 @@ int32_t ls_test_tblock(const void* att, float* u, const void* wo, const void* w1
     else
       ls::require(ls::make_tile_map(&m.tail_out, tail_out, 2, 256, R, 128), "tensor map tail", LS_ERR_CUDA);
     ls::TBlockParams p{};
-    p.R = R, p.T = T, p.lengths = lengths, p.vec = vec, p.tail_mode = tail_mode;
+    p.R = R, p.T = T, p.lengths = lengths, p.vec = vec, p.tail_mode = tail_mode, p.fp16 = fp16, p.no_skip = no_skip;
     LS_CUDA(ls::launch_tblock(m, p, sms, (cudaStream_t)stream, plan_out));
+  });
+}
+
+int32_t ls_test_groupnorm_mish(const float* x, void* stats, const float* gamma, const float* beta, const float* temb,
+                               int64_t temb_bstride, const float* addend, float* out_f32, void* out_h, int32_t B,
+                               int32_t C, int32_t T, int32_t G, const int32_t* lengths, int32_t fp16, void* stream) {
+  return ls::guarded([&] {
+    ls::require(x && stats && gamma && beta, "ls_test_groupnorm_mish: null argument");
+    LS_CUDA(ls::launch_groupnorm_mish(x, reinterpret_cast<float2*>(stats), gamma, beta, temb, temb_bstride, addend, out_f32,
+                                      reinterpret_cast<__nv_bfloat16*>(out_h), B, C, T, G, lengths, fp16,
+                                      (cudaStream_t)stream));
   });
 }
 

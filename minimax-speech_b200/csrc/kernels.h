@@ -237,7 +237,8 @@ cudaError_t launch_mask_to_lengths(const float* mask, int* lengths, int B, int T
                                    int* bad_flag = nullptr);
 // GroupNorm(G) + Mish on time-major fp32 x [B][T][C] with per-row statistics over the valid frames (the non-causal
 // ConditionalDecoder's blocks): stats [B][G] scratch; then + temb[b] (optional) + addend (optional fp32, same layout);
-// fp32 and / or 16-bit outputs (either may be null); padding rows come out as 0 (+ temb + addend).
+// fp32 and / or 16-bit outputs (either may be null); padding rows come out as exactly 0 (temb and addend are not added
+// there).  Lengths above T count as T.
 cudaError_t launch_groupnorm_mish(const float* x, float2* stats, const float* gamma, const float* beta, const float* temb,
                                   long long temb_bstride, const float* addend, float* out_f32, __nv_bfloat16* out_h, int B,
                                   int C, int T, int G, const int* lengths, int fp16, cudaStream_t s);

@@ -23,7 +23,8 @@ EXPORTS = ["ls_abi_version", "ls_last_error", "ls_device_check", "ls_flow_create
            "ls_flow_destroy",
            "ls_flow_estimator_forward", "ls_flow_solve", "ls_dac_create", "ls_dac_destroy", "ls_dac_hop_length",
            "ls_dac_decode", "ls_synthesize_host", "ls_fsq_encode", "ls_mask_to_lengths", "ls_graph_create", "ls_graph_buffer",
-           "ls_graph_launch", "ls_graph_kernel_count", "ls_graph_destroy", "ls_launch_count", "ls_debug_set_buffer", "ls_profile_begin", "ls_profile_end", "ls_test_conv_gemm", "ls_test_attention", "ls_test_tblock"]
+           "ls_graph_launch", "ls_graph_kernel_count", "ls_graph_destroy", "ls_launch_count", "ls_debug_set_buffer", "ls_profile_begin", "ls_profile_end", "ls_test_conv_gemm", "ls_test_attention", "ls_test_tblock",
+           "ls_test_groupnorm_mish"]
 
 
 class LsTensor(C.Structure):
@@ -51,6 +52,10 @@ class ConvGemmDesc(C.Structure):
         ("out_ld", C.c_int64), ("out_shift", C.c_int64), ("out_bstride", C.c_int64), ("out_alloc", C.c_int64),
         ("out_valid_mul", C.c_int64),
         ("fp16", C.c_int32),  # 0 (the default of a fresh descriptor): bf16 operands; 1: fp16
+        ("zero_skipped", C.c_int32),
+        # fused residual GEMM (res_w set): a 1x1 convolution of res_a0 (| res_a1) added in the epilogue
+        ("res_a0", C.c_void_p), ("res_a1", C.c_void_p), ("res_a0_C", C.c_int32), ("res_a1_C", C.c_int32),
+        ("res_w", C.c_void_p), ("res_K", C.c_int32), ("res_bias", C.c_void_p),
     ]
 
 
@@ -146,7 +151,8 @@ def load():
         lib.ls_graph_destroy.restype = None
         lib.ls_debug_set_buffer.argtypes = [vp, i64]
         lib.ls_profile_end.argtypes = [C.POINTER(ProfileEntry), i32]
-        lib.ls_test_tblock.argtypes = [vp] * 10 + [i32, i32, i32, i32, vp, vp]
+        lib.ls_test_tblock.argtypes = [vp] * 10 + [i32, i32, i32, i32, i32, i32, vp, vp]
+        lib.ls_test_groupnorm_mish.argtypes = [vp, vp, vp, vp, vp, i64, vp, vp, vp, i32, i32, i32, i32, vp, i32, vp]
         lib.ls_test_conv_gemm.argtypes = [C.POINTER(ConvGemmDesc), i32, vp, vp]
         lib.ls_test_attention.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp, i64, i64, vp]
         for name in EXPORTS:
@@ -155,7 +161,7 @@ def load():
                 fn.restype = i32
         # the kernel test hooks' SM count and plan arguments (just before the stream) are optional for Python callers
         lib.ls_test_conv_gemm = _plan_args_optional(lib.ls_test_conv_gemm, 1)
-        lib.ls_test_tblock = _plan_args_optional(lib.ls_test_tblock, 13)
+        lib.ls_test_tblock = _tblock_args_optional(lib.ls_test_tblock)
         # ... and so are the attention hook's fp16 flag and bias arguments (bf16, no bias)
         lib.ls_test_attention = _attention_args_optional(lib.ls_test_attention)
         _lib = lib
@@ -167,6 +173,19 @@ def _plan_args_optional(fn, n_fixed):
     def call(*args):
         if len(args) == n_fixed + 1:
             args = args[:-1] + (0, None, args[-1])
+        return fn(*args)
+    call.__name__ = fn.__name__
+    return call
+
+
+def _tblock_args_optional(fn):
+    """fn(13 fixed, fp16, no_skip, num_sms, plan_out, stream) also callable as fn(13 fixed, num_sms, plan_out, stream) and
+    fn(13 fixed, stream): bf16 operands, padding-only tiles skipped (and the device's SM count, no plan)"""
+    def call(*args):
+        if len(args) == 14:
+            args = args[:-1] + (0, None, args[-1])
+        if len(args) == 16:
+            args = args[:13] + (0, 0) + args[13:]
         return fn(*args)
     call.__name__ = fn.__name__
     return call

@@ -48,6 +48,12 @@ BARS = {
                             # does, and a last-bit difference in the fp32 statistics flips single roundings (measured 9.9e-5)
     "tblock_qkv": 4e-3,     # QKV of bf16(LayerNorm(u'')), bf16 output (measured 1.8e-3)
     "tblock_tail": 4e-3,    # bf16 copy of u'' (measured 1.7e-3)
+    # the same outputs with fp16 operands (fp32 outputs keep the bars above)
+    "ln_f16": 6e-4,         # fp16 of a LayerNorm output (measured 2.1e-4: the fp16 rounding itself)
+    "mish_f16": 6e-4,       # fp16 of a LayerNorm + Mish output (measured 2.1e-4)
+    "tblock_u_f16": 7.5e-5, # u'' with the reference's fp16 roundings of n3 and h (measured 3.2e-5)
+    "tblock_qkv_f16": 6e-4, # QKV of fp16(LayerNorm(u'')), fp16 output (measured 2.4e-4)
+    "tblock_tail_f16": 6e-4,  # fp16 copy of u'' (measured 2.1e-4)
 }
 
 _measured = {}  # bar name -> worst per-tile error seen (printed at the end of the module)
@@ -69,6 +75,10 @@ def bf16(t):
     return t.to(torch.bfloat16)
 
 
+# the 16-bit operand format of a launch: dtype, rounding, the fp16 flag of the hooks, the suffix of its bar names
+H16 = {"bf16": (torch.bfloat16, bf16, 0, ""), "fp16": (torch.float16, lambda t: t.half(), 1, "_f16")}
+
+
 def bits(t):
     return t.view(torch.int32) if t.dtype == torch.float32 else t.view(torch.int16)
 
@@ -81,13 +91,14 @@ def plan_dict(plan):
 def conv_gemm(a0, w, num_sms, *, M=None, block_n=None, dil=1, pad=0, lengths=None, m_len_mul=1, m_len_add=0,
               skip_halo=0, chan_mod=None, bias=None, act=0, ln=None, temb=None, addend=None, out0=None, out1=None,
               out1_mode=0, p1=None, n_store=None, out_ld=None, out_shift=0, out_bstride=None, out_alloc=None,
-              out_valid_mul=None):
-    """a0 [B,T,C] bf16, w [taps,N,K] bf16; returns the plan the launch used."""
+              out_valid_mul=None, a1=None, res=None, zero_skipped=0, fp16=0):
+    """a0 [B,T,C0] (+ a1 [B,T,C1], the K split) bf16, w [taps,N,K] bf16 (fp16 = 1: both fp16); res = (res_a0,
+    res_a1 or None, res_w [N][res_K], res_bias or None): the fused residual GEMM.  Returns the plan the launch used."""
     B, T_in, C0 = a0.shape
     taps, N, K = w.shape
     d = native.ConvGemmDesc()
     d.a0, d.a0_C, d.T_in = native.ptr(a0), C0, T_in
-    d.a1, d.a1_C = C.c_void_p(0), 0
+    d.a1, d.a1_C = native.ptr(a1), (a1.shape[2] if a1 is not None else 0)
     d.w, d.K = native.ptr(w), K
     d.B, d.M, d.N = B, M or T_in, N
     d.block_n = block_n or N
@@ -111,6 +122,14 @@ def conv_gemm(a0, w, num_sms, *, M=None, block_n=None, dil=1, pad=0, lengths=Non
     d.out_bstride = out_bstride if out_bstride is not None else d.M * d.out_ld
     d.out_alloc = out_alloc if out_alloc is not None else d.M * d.out_ld
     d.out_valid_mul = out_valid_mul if out_valid_mul is not None else d.out_ld
+    d.zero_skipped = zero_skipped
+    if fp16:  # (a descriptor may already come with fp16 = 1)
+        d.fp16 = 1
+    if res is not None:
+        ra0, ra1, rw, rbias = res
+        d.res_a0, d.res_a0_C = native.ptr(ra0), (ra0.shape[2] if ra0 is not None else 0)
+        d.res_a1, d.res_a1_C = native.ptr(ra1), (ra1.shape[2] if ra1 is not None else 0)
+        d.res_w, d.res_K, d.res_bias = native.ptr(rw), rw.shape[1], native.ptr(rbias)
     plan = (C.c_int32 * 8)()
     native.check(native.load().ls_test_conv_gemm(C.byref(d), num_sms, plan, native.current_stream_ptr(DEV)),
                  "ls_test_conv_gemm")
@@ -142,10 +161,11 @@ def mish(x):
 class Geometry:
     """Where every element of one output of a conv_gemm launch comes from.  Output element f (flat index inside a
     batch item) is GEMM element (q, n) with q * out_ld + n + out_shift = f; its tile is (b, q // 128, n // block_n).
-    state: 2 = stored value, 1 = zero (padding inside a processed tile), 0 = never written (keeps its initial bits)."""
+    state: 2 = stored value, 1 = zero (padding inside a processed tile, or every stored position of a skipped tile when
+    the launch has zero_skipped = 1), 0 = never written (keeps its initial bits)."""
 
     def __init__(self, shape, B, M, N, block_n, lengths, m_len_mul=1, m_len_add=0, skip_halo=0, n_store=None,
-                 out_ld=None, out_shift=0, out_valid_mul=None):
+                 out_ld=None, out_shift=0, out_valid_mul=None, zero_skipped=0):
         out_ld = out_ld or N
         n_store = n_store or N
         out_valid_mul = out_valid_mul if out_valid_mul is not None else out_ld
@@ -163,7 +183,8 @@ class Geometry:
         skipped = (mt[None] * 128) >= (lens[:, None] * m_len_mul + m_len_add + skip_halo)
         valid = f[None] < (lens[:, None] * out_valid_mul)
         state = torch.where(valid, 2, 1)
-        state = torch.where(skipped | ~produced[None], 0, state)
+        state = torch.where(skipped, 1 if zero_skipped else 0, state)
+        state = torch.where(~produced[None], 0, state)
         self.shape = shape
         self.tile = tile.view(shape)
         self.state = state.view(shape).to(torch.int8)
@@ -366,48 +387,56 @@ def test_resident_conv1_inplace_f16_residual_snake():
 
 def test_streamed_qkv_linear_several_n_tiles():
     """QKV-style linear K 256 -> N 1536 in 256-wide tiles (512 TMEM columns): streamed weights, one issuer, several N
-    tiles and several tiles per CTA; out1 = bf16 of the accumulator."""
+    tiles and several tiles per CTA; out1 = 16-bit copy of the accumulator (1 ulp), with bf16 and with fp16 operands."""
     B, M, K, N = 3, 300, 256, 1536
 
-    def case():
-        rn = _gen(400)
-        a = bf16(rn(B, M, K))
-        w = bf16(rn(1, N, K, scale=K ** -0.5))
-        lengths = _lens([300, 0, 77])
-        geo = Geometry((B, M, N), B, M, N, 256, lengths)
-        return dict(name="qkv linear 256->1536",
-                    launch=dict(a0=a, w=w, block_n=256, lengths=lengths, out1_mode=native.OUT1_COPY),
-                    outputs={"out1": (_nan(B, M, N, dtype=torch.bfloat16), geo, "ulp", conv64(a, w, 1, 0),
-                                      conv64(a.abs(), w.abs(), 1, 0))})
+    def make_case(precision):
+        dt, r16, fp16, _ = H16[precision]
+
+        def case():
+            rn = _gen(400)
+            a = r16(rn(B, M, K))
+            w = r16(rn(1, N, K, scale=K ** -0.5))
+            lengths = _lens([300, 0, 77])
+            geo = Geometry((B, M, N), B, M, N, 256, lengths)
+            return dict(name=f"qkv linear 256->1536 {precision}",
+                        launch=dict(a0=a, w=w, block_n=256, lengths=lengths, out1_mode=native.OUT1_COPY, fp16=fp16),
+                        outputs={"out1": (_nan(B, M, N, dtype=dt), geo, "ulp", conv64(a, w, 1, 0),
+                                          conv64(a.abs(), w.abs(), 1, 0))})
+        return case
 
     def expect(sms, geo):
         return dict(dual=0, b_resident=0, a_stages=3, b_stages=3, tma_out=1)
-    plans = run_conv_case(case, [0, 1, 2, 5, 7], expect)
-    assert max(p["tiles_per_cta"] for _, p, _ in plans) >= 2
+    for precision in ("bf16", "fp16"):
+        plans = run_conv_case(make_case(precision), [0, 1, 2, 5, 7], expect)
+        assert max(p["tiles_per_cta"] for _, p, _ in plans) >= 2
 
 
-@pytest.mark.parametrize("variant", ["temb_copy", "addend_ln"])
-def test_layernorm_epilogues_multi_tile(variant):
+@pytest.mark.parametrize("variant,precision", [("temb_copy", "bf16"), ("addend_ln", "bf16"), ("temb_copy", "fp16"),
+                                               ("addend_ln", "fp16")],
+                         ids=["temb_copy", "addend_ln", "temb_copy-fp16", "addend_ln-fp16"])
+def test_layernorm_epilogues_multi_tile(variant, precision):
     """Flow-estimator resnet conv (k = 3, pad 2) with the LayerNorm + Mish epilogue over several tiles per CTA: the
-    statistics area alternates with the tile parity.  temb_copy: + time embedding -> bf16 copy; addend_ln: + fp32
-    residual -> fp32 out0 and bf16 LayerNorm of it."""
+    statistics area alternates with the tile parity.  temb_copy: + time embedding -> 16-bit copy; addend_ln: + fp32
+    residual -> fp32 out0 and 16-bit LayerNorm of it.  bf16 or fp16 operands and 16-bit outputs."""
     B, M, K, N = 3, 333, 320, 256
+    dt, r16, fp16, sfx = H16[precision]
 
     def case():
         rn = _gen(500 + len(variant))
-        a = bf16(rn(B, M, K))
-        w = bf16(rn(3, N, K, scale=(3 * K) ** -0.5))
+        a = r16(rn(B, M, K))
+        w = r16(rn(3, N, K, scale=(3 * K) ** -0.5))
         bias = rn(N, scale=0.1)
         lg, lb = 1 + rn(N, scale=0.1), rn(N, scale=0.1)
         lengths = _lens([333, 0, 200])
         geo = Geometry((B, M, N), B, M, N, N, lengths)
         y = mish(F.layer_norm(conv64(a, w, 1, 2) + bias.double(), (N,), lg.double(), lb.double(), 1e-5))
-        kw = dict(a0=a, w=w, pad=2, lengths=lengths, bias=bias, act=native.ACT_LN_MISH, ln=(lg, lb))
+        kw = dict(a0=a, w=w, pad=2, lengths=lengths, bias=bias, act=native.ACT_LN_MISH, ln=(lg, lb), fp16=fp16)
         if variant == "temb_copy":
             temb = rn(B, N)
             y = y + temb.double()[:, None, :]
             kw.update(temb=temb, out1_mode=native.OUT1_COPY)
-            outputs = {"out1": (_nan(B, M, N, dtype=torch.bfloat16), geo, "mish_bf16", y, None)}
+            outputs = {"out1": (_nan(B, M, N, dtype=dt), geo, "mish_bf16" if not fp16 else "mish_f16", y, None)}
         else:
             addend = rn(B, M, N)
             g2, b2 = 1 + rn(N, scale=0.1), rn(N, scale=0.1)
@@ -415,8 +444,8 @@ def test_layernorm_epilogues_multi_tile(variant):
             y1 = F.layer_norm(y, (N,), g2.double(), b2.double(), 1e-5)
             kw.update(addend=addend, out1_mode=native.OUT1_LN, p1=(g2, b2))
             outputs = {"out0": (_nan(B, M, N), geo, "ln_mish_f32", y, None),
-                       "out1": (_nan(B, M, N, dtype=torch.bfloat16), geo, "ln_bf16", y1, None)}
-        return dict(name=f"resnet conv3 LN+Mish {variant}", launch=kw, outputs=outputs)
+                       "out1": (_nan(B, M, N, dtype=dt), geo, "ln_bf16" if not fp16 else "ln_f16", y1, None)}
+        return dict(name=f"resnet conv3 LN+Mish {variant} {precision}", launch=kw, outputs=outputs)
 
     def expect(sms, geo):
         return dict(dual=0, b_resident=0, a_stages=2, b_stages=3, tma_out=1)
@@ -539,23 +568,25 @@ def test_conv_hook_refuses_sm_counts_outside_the_device():
 
 
 # ------------------------------------------------------------------------------------------ fused transformer block
-def _tblock_operands(R, seed):
+def _tblock_operands(R, seed, r16=bf16):
     rn = _gen(seed)
-    att = bf16(rn(R, 512))
+    att = r16(rn(R, 512))
     u = rn(R, 256, scale=2.0) + 0.5
-    wo = bf16(rn(256, 512, scale=512 ** -0.5))
-    w1 = bf16(rn(1024, 256, scale=256 ** -0.5))
-    w2 = bf16(rn(256, 1024, scale=1024 ** -0.5))
-    wqkv = bf16(rn(1536, 256, scale=256 ** -0.5))
+    wo = r16(rn(256, 512, scale=512 ** -0.5))
+    w1 = r16(rn(1024, 256, scale=256 ** -0.5))
+    w2 = r16(rn(256, 1024, scale=1024 ** -0.5))
+    wqkv = r16(rn(1536, 256, scale=256 ** -0.5))
     vec = torch.cat([rn(256, scale=0.1), 1 + rn(256, scale=0.1), rn(256, scale=0.1), rn(1024, scale=0.2),
                      rn(256, scale=0.1), 1 + rn(256, scale=0.1), rn(256, scale=0.1)]).contiguous()
     return att, u, wo, w1, w2, wqkv, vec
 
 
-def _tblock_ref64(att, u, wo, w1, w2, wqkv, vec, head):
-    """float64, with the kernel's bf16 roundings of the FF input, the GELU output and the QKV input"""
+def _tblock_ref64(att, u, wo, w1, w2, wqkv, vec, head, r16=bf16):
+    """float64, with the kernel's 16-bit roundings (r16: bf16 or fp16) of the FF input, the GELU output and the QKV
+    input"""
     d = lambda t: t.double()
-    r16 = lambda t: bf16(t.float()).double()
+    rnd = r16
+    r16 = lambda t: rnd(t.float()).double()
     bo, g3, be3, b1, b2, g1n, be1n = [d(v) for v in torch.split(vec, [256, 256, 256, 1024, 256, 256, 256])]
     if head:
         u2 = d(u)
@@ -568,16 +599,16 @@ def _tblock_ref64(att, u, wo, w1, w2, wqkv, vec, head):
     return u2, n1 @ d(wqkv).T
 
 
-def _tblock_launch(ops, u, tail_mode, lengths, T, num_sms):
+def _tblock_launch(ops, u, tail_mode, lengths, T, num_sms, fp16=0, no_skip=0):
     att, _, wo, w1, w2, wqkv, vec = ops
     R = att.shape[0]
-    qkv = _nan(R, 1536, dtype=torch.bfloat16) if tail_mode != 1 else None
-    tail = _nan(R, 256, dtype=torch.bfloat16) if tail_mode == 1 else None
+    qkv = _nan(R, 1536, dtype=att.dtype) if tail_mode != 1 else None
+    tail = _nan(R, 256, dtype=att.dtype) if tail_mode == 1 else None
     plan = (C.c_int32 * 2)()
     native.check(native.load().ls_test_tblock(native.ptr(att), native.ptr(u), native.ptr(wo), native.ptr(w1),
                                               native.ptr(w2), native.ptr(wqkv), native.ptr(vec), native.ptr(qkv),
-                                              native.ptr(tail), native.ptr(lengths), R, T, tail_mode, num_sms, plan,
-                                              native.current_stream_ptr(DEV)), "ls_test_tblock")
+                                              native.ptr(tail), native.ptr(lengths), R, T, tail_mode, fp16, no_skip,
+                                              num_sms, plan, native.current_stream_ptr(DEV)), "ls_test_tblock")
     torch.cuda.synchronize()
     return qkv, tail, (plan[0], plan[1])
 
@@ -603,56 +634,70 @@ def _tile_rel(out, ref, rows_mask, col_block):
 TB_T, TB_LENS, TB_SMS = 700, [700, 0, 130, 450, 690], [0, 1, 3, 5, 7, 14]
 
 
-@pytest.mark.parametrize("tail_mode", [0, 1, 2])
-def test_tblock_plans_bitwise_and_per_tile(tail_mode):
+def tblock_plans(tail_mode, precision="bf16", no_skip=0):
+    """Every SM count of TB_SMS: the plan, the initial bits of what a launch must not write, per-tile errors against
+    float64 (bars tblock_* with the precision's suffix) and bitwise identity across the SM counts.  no_skip = 1: every
+    tile is processed, padding rows included (row-local reference there, a zero tail).  Returns the outputs of the
+    first launch (u, qkv, tail) and the row masks (valid, in_real)."""
+    dt, r16, fp16, sfx = H16[precision]
     R = TB_T * len(TB_LENS)
     n_tiles = -(-R // 128)
-    ops = _tblock_operands(R, 900 + tail_mode)
+    ops = _tblock_operands(R, 900 + tail_mode, r16)
     lengths = _lens(TB_LENS)
-    u_ref, qkv_ref = _tblock_ref64(*ops, head=tail_mode == 2)
+    u_ref, qkv_ref = _tblock_ref64(*ops, head=tail_mode == 2, r16=r16)
     row = torch.arange(R, device=DEV)
     valid = (row % TB_T) < lengths.long()[row // TB_T]
     tile_real = torch.stack([valid[t * 128:(t + 1) * 128].any() for t in range(n_tiles)])
-    in_real = tile_real[row // 128]  # rows of tiles that are processed
     assert not bool(tile_real.all()) and bool(tile_real[-1])
+    if no_skip:
+        tile_real = torch.ones_like(tile_real)
+    in_real = tile_real[row // 128]  # rows of tiles that are processed
     first = None
     all_reals = []
     for sms in TB_SMS:
         u = ops[1].clone()
-        qkv, tail, (grid, tpc) = _tblock_launch(ops, u, tail_mode, lengths, TB_T, sms)
+        qkv, tail, (grid, tpc) = _tblock_launch(ops, u, tail_mode, lengths, TB_T, sms, fp16, no_skip)
         n = sms if sms else SMS
         reals = [int(tile_real[c::grid].sum()) for c in range(grid)]
         all_reals += reals if tpc >= 2 else []
-        print(f"  tblock tail_mode={tail_mode} sms={n:3d} grid={grid} tiles_per_cta={tpc}"
+        print(f"  tblock tail_mode={tail_mode} {precision} no_skip={no_skip} sms={n:3d} grid={grid} tiles_per_cta={tpc}"
               f"  real tiles per CTA: min {min(reals)} max {max(reals)}")
         assert (grid, tpc) == (min(n_tiles, n), -(-n_tiles // min(n_tiles, n)))
         # rows of skipped tiles keep their initial bits; u is only written in tail_mode 0
         if tail_mode == 0:
             assert torch.equal(bits(u)[~in_real], bits(ops[1])[~in_real])
             e = _tile_rel(u, u_ref, in_real, 256)
-            _note("tblock_u", e)
-            assert e <= BARS["tblock_u"], (sms, e)
+            _note("tblock_u" + sfx, e)
+            assert e <= BARS["tblock_u" + sfx], (sms, e)
         else:
             assert torch.equal(bits(u), bits(ops[1]))
         if tail_mode != 1:
-            assert bool(qkv[~in_real].isnan().all())
+            assert bool(qkv[~in_real].isnan().all()) and not bool(qkv[in_real].isnan().any())
             e = _tile_rel(qkv, qkv_ref, in_real, 128)
-            _note("tblock_qkv", e)
-            assert e <= BARS["tblock_qkv"], (sms, e)
+            _note("tblock_qkv" + sfx, e)
+            assert e <= BARS["tblock_qkv" + sfx], (sms, e)
             res = [bits(qkv)] + ([bits(u)] if tail_mode == 0 else [])
         else:
-            assert bool(tail[~in_real].isnan().all())
+            assert bool(tail[~in_real].isnan().all()) and not bool(tail[in_real].isnan().any())
             assert bool((bits(tail)[in_real & ~valid] == 0).all())  # padding rows of processed tiles: zero
             e = _tile_rel(tail, u_ref, valid, 256)
-            _note("tblock_tail", e)
-            assert e <= BARS["tblock_tail"], (sms, e)
+            _note("tblock_tail" + sfx, e)
+            assert e <= BARS["tblock_tail" + sfx], (sms, e)
             res = [bits(tail)]
         if first is None:
             first = [r.clone() for r in res]
+            outs = (u, qkv, tail)
         else:
             for a_, b_ in zip(res, first):
-                assert torch.equal(a_, b_), f"tblock tail_mode={tail_mode}: sms={n} differs bitwise"
-    assert 0 in all_reals and 1 in all_reals and any(r >= 3 for r in all_reals)
+                assert torch.equal(a_, b_), f"tblock tail_mode={tail_mode} {precision}: sms={n} differs bitwise"
+    if not no_skip:
+        assert 0 in all_reals and 1 in all_reals and any(r >= 3 for r in all_reals)
+    return outs, valid, in_real
+
+
+@pytest.mark.parametrize("tail_mode", [0, 1, 2])
+def test_tblock_plans_bitwise_and_per_tile(tail_mode):
+    tblock_plans(tail_mode)
 
 
 def test_tblock_grid_follows_num_sms_on_every_call():
